@@ -22,6 +22,10 @@ over the ranks, K all-gathered over NCCL and mirrored (strong scaling: the total
            peak measured live by gprb_fp64_dmma_peak (MEASURED_PEAKS.json carries no fp64 entry).
   cpu_baseline: the UNMODIFIED reference C++ (oracle/_ref) on a bounded sample of the same workload,
            row-split over the host cores like the reference's MPI split.
+
+--dump-outputs DIR writes what the timed calls returned in their last step as DIR/<name>.npy (float64), so that two
+builds can be compared output by output on identical (seeded) inputs: a fixed sample of K and dK/dl (rows = columns =
+K_sample_index), the LML and its gradient of the end-to-end leg, and the predictions of a fixed sample of structures.
 """
 import argparse
 import json
@@ -58,6 +62,25 @@ SO3_CPU_SECONDS = []     # numpy port of SO3.calculate (oracle/so3.py), seconds 
 
 def flops_of(p_ff, p_ef, p_ee, d=D):
     return 32.0 * d * p_ff + 8.0 * d * p_ef + 2.0 * d * p_ee
+
+
+# --dump-outputs: K and dK/dl of S5 are 77 GB each, so a fixed sample of rows (= columns) is written (about 20 MB in all)
+DUMP_K_ROWS, DUMP_K_ENERGY_ROWS, DUMP_STRUCTURES = 1024, 128, 1024
+
+
+def k_sample_index(NE, N):
+    """Sorted, seeded row (= column) indices of the N x N covariance: up to DUMP_K_ENERGY_ROWS energy rows, the rest
+    force rows, so that the sample holds parts of the EE, EF and FF blocks and their diagonals."""
+    rng = np.random.default_rng(0)
+    n_e = min(NE, DUMP_K_ENERGY_ROWS)
+    n_f = min(N - NE, DUMP_K_ROWS - n_e)
+    return np.sort(np.concatenate([rng.choice(NE, n_e, replace=False), NE + rng.choice(N - NE, n_f, replace=False)]))
+
+
+def dump(dir_, name, a):
+    if dir_ is not None:
+        os.makedirs(dir_, exist_ok=True)
+        np.save(os.path.join(dir_, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -346,7 +369,8 @@ def small_n_block(des):
             model["db_filename"] = db
             with open(js, "w") as fp:
                 json.dump(model, fp)
-            with contextlib.redirect_stdout(io.StringIO()):
+            # GP.load opens the default log file gpr.log in the working directory: keep it in the temporary one
+            with contextlib.redirect_stdout(io.StringIO()), contextlib.chdir(tmp):
                 gp = GP.load(js)
         gp.log_file = None
         theta = np.array(gp.kernel.parameters())
@@ -454,10 +478,15 @@ def main():
     ap.add_argument("--s4-maxiter", type=int, default=10)
     ap.add_argument("--s4-budget-s", type=float, default=400.0, help="wall budget of the S4 GP.fit (no new LML evaluation after it)")
     ap.add_argument("--profile-e2e", default=None, help="write a cProfile listing of one end-to-end step to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    dump_dir = args.dump_outputs if rank == 0 else None
     n_struct, nrep, seed0, desc = WORKLOADS[args.workload]
     threads = os.cpu_count() or 1
     config = {"workload": desc, "kernel": "RBF zeta=2 sigma=%g l=%g" % (SIGMA, ELL), "descriptor": "SO3 nmax=3 lmax=4 rcut=5.0 (d=30)",
@@ -557,12 +586,23 @@ def main():
     t_wall0 = time.time()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
+    out = None
     for _ in range(args.steps):
+        out = None            # free the previous K and dK/dl before the next build allocates its own
         out = step()
-        del out
     ev1.record()
     barrier()
     t_wall1 = time.time()
+    if dump_dir is not None:
+        K_last, dK_last, _ = out
+        idx = k_sample_index(NE, N)
+        idx_dev = torch.as_tensor(idx, device="cuda")
+        dump(dump_dir, "K_sample_index", idx)
+        dump(dump_dir, "K_sample", K_last.index_select(0, idx_dev).index_select(1, idx_dev).cpu().numpy())
+        if world == 1:        # with several ranks dK/dl holds this rank's rows only, and their windows adapt per build
+            dump(dump_dir, "dK_dl_sample", dK_last.index_select(0, idx_dev).index_select(1, idx_dev).cpu().numpy())
+        del K_last, dK_last
+    del out
     prof, _lib.PROFILE = _lib.PROFILE, None
     launches = lib.gprb_launch_count() - launches0
     ms_step = ev0.elapsed_time(ev1) / args.steps
@@ -661,6 +701,8 @@ def main():
         # device -> host reads of a step: gprb_lml_eval copies 9 doubles + 2 status words back, once
         d2h = 80 * sum(1 for n, _, _, _ in prof if n == "gprb_lml_eval") / args.steps
         lml, grad = res
+        dump(dump_dir, "lml", [lml])
+        dump(dump_dir, "lml_grad", grad)
         result["e2e"] = {"value": flops / dt * 1e-9, "unit": "GFLOP/s", "h2d_bytes_per_step": int(h2d),
                          "d2h_bytes_per_step": int(d2h), "ms_per_step": dt * 1e3,
                          "ms_per_step_min_max_on_rank0": [min(step_s) * 1e3, max(step_s) * 1e3],
@@ -715,6 +757,11 @@ def main():
             dF = max(float(np.abs(res[k][1] - singles[k][1]).max()) for k in range(8))
             dS = max(max(abs(res[k][3] - singles[k][3]), float(np.abs(res[k][4] - singles[k][4]).max())) for k in range(8))
             assert len(res) == n_test and dE <= 1e-8 and dF <= 1e-8, (dE, dF)
+            if dump_dir is not None:
+                pick = np.sort(np.random.default_rng(1).choice(n_test, min(n_test, DUMP_STRUCTURES), replace=False))
+                for name, k in (("predict_energy", 0), ("predict_forces", 1), ("predict_energy_std", 3), ("predict_forces_std", 4)):
+                    dump(dump_dir, name, np.stack([res[i][k] for i in pick]))
+                dump(dump_dir, "predict_index", pick)
             # conditioning diagnostic: how far the reference's explicit-inverse variance formula is from the factor route
             from gpr_calculator_b200.batch import rows_from_batch
             E_t, F_t = rows_from_batch(des.calculate_batch(tests[:2], to_host=False), None)

@@ -374,7 +374,9 @@ __global__ void __launch_bounds__(BIG ? BIG_WARPS * 32 : THREADS, NB == 0 ? 2 : 
                     }
                 }
             } else if (EE) {
-                // K_ee[I, J] = 1 / (n_I n_J) sum k   (rbf_kernel.py:56-70, dot_kernel.py:46); symmetric mode mirrors
+                // K_ee[I, J] = 1 / (n_I n_J) sum k   (rbf_kernel.py:56-70, dot_kernel.py:46).  Symmetric mode writes
+                // J >= I only and gprb_kee mirrors afterwards: a group split over three or more CTAs is summed by
+                // atomics in arrival order, which can differ between K[I, J] and K[J, I] in the last bits.
                 const double nn = (double)P.group_rowsA[I] * (double)P.group_rowsB[J];
                 const double val = nn > 0 ? v / nn : 0.0;
                 double *dst = isgrad ? P.dK : P.K;
@@ -382,10 +384,6 @@ __global__ void __launch_bounds__(BIG ? BIG_WARPS * 32 : THREADS, NB == 0 ? 2 : 
                 if (!(P.mode == GPRB_FF_SYMMETRIC && J < I)) {
                     double *qd = dst + (long long)(I - P.grp_begin) * ld + J;
                     if (shared) atomicAdd(qd, val); else *qd = val;
-                    if (P.mode == GPRB_FF_SYMMETRIC && J > I) {
-                        double *qt = dst + (long long)J * ld + I;
-                        if (shared) atomicAdd(qt, val); else *qt = val;
-                    }
                 }
             } else {
                 // a side = force group I (window), b side = energy group J; K_ef = -(1/n_J) sum
@@ -944,10 +942,14 @@ extern "C" int gprb_kee(int kernel, const gprb_pack *e1_, const gprb_pack *e2, d
     P.group_rowsA = e1->d_group_rows;
     P.n_groupsB = e2->n_groups; P.ks = e1->ks;
     P.win_r0 = e1->row_ptr[grp_begin]; P.win_r1 = e1->row_ptr[grp_end];
-    // the training block is symmetric: evaluate the J >= I group pairs once and write both entries
+    // the training block is symmetric: evaluate the J >= I group pairs once, then mirror them
     P.mode = (e1 == e2 && grp_begin == 0 && grp_end == e1->n_groups) ? GPRB_FF_SYMMETRIC : GPRB_FF_FULL;
     P.grp_begin = grp_begin;
     P.K = K; P.ldk = ldk; P.dK = dK; P.lddk = lddk;
     P.n_splits = choose_splits(e1->sched_n, e2->n_groups);
-    return dispatch_cov<0>(kernel, dK != nullptr, P, e1->sched_n, st);
+    rc = dispatch_cov<0>(kernel, dK != nullptr, P, e1->sched_n, st);
+    if (rc || P.mode != GPRB_FF_SYMMETRIC) return rc;
+    rc = gprb_symmetrize(K, ldk, e1->n_groups, st);
+    if (rc == GPRB_OK && dK) rc = gprb_symmetrize(dK, lddk, e1->n_groups, st);
+    return rc;
 }

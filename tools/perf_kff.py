@@ -1,6 +1,6 @@
 """Quick device timing of gprb_kff on random packed rows shaped like the S5 config (dev tool)."""
-import sys, json
-sys.path.insert(0, '/root/repo')
+import os, sys, json
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from gpr_calculator_b200 import _lib
 from gpr_calculator_b200.device import Pack, empty, ptr, stream, c_vp

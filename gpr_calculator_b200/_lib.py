@@ -44,17 +44,10 @@ SIGNATURES = {
     "gprb_kee_diag": (c_int, [c_int, c_vp, c_dbl, c_dbl, c_dbl, c_vp, c_vp]),
     "gprb_add_noise": (c_int, [c_vp, c_ll, c_int, c_int, c_dbl, c_dbl, c_vp]),
     "gprb_chol_factor": (c_int, [c_vp, c_ll, c_int, c_vp]),
-    "gprb_chol_solve_vec": (c_int, [c_vp, c_ll, c_int, c_vp, c_vp]),
-    "gprb_chol_inverse": (c_int, [c_vp, c_ll, c_int, c_vp, c_ll, c_vp]),
-    "gprb_lml_terms": (c_int, [c_vp, c_ll, c_int, c_vp, c_vp, c_vp, c_vp]),
-    "gprb_lml_grad_trace": (c_int, [c_int, c_int, c_int, c_vp, c_vp, c_ll, c_vp, c_ll, c_int, c_dbl, c_dbl, c_int, c_vp, c_vp]),
     "gprb_chol_inverse_rows": (c_int, [c_vp, c_ll, c_int, c_int, c_int, c_int, c_vp, c_ll, c_vp]),
-    "gprb_lml_grad_trace_rows": (c_int, [c_int, c_int, c_int, c_vp, c_vp, c_ll, c_int, c_vp, c_ll, c_vp, c_ll,
-                                         c_int, c_dbl, c_dbl, c_vp, c_vp]),
     "gprb_symmetrize": (c_int, [c_vp, c_ll, c_int, c_vp]),
     "gprb_transpose_copy": (c_int, [c_vp, c_ll, c_vp, c_ll, c_int, c_int, c_vp]),
     "gprb_fp64_dmma_peak": (c_int, [c_vp, c_vp]),
-    "gprb_w_block_sum": (c_int, [c_int, c_int, c_int, c_int, c_int, c_vp, c_vp, c_ll, c_vp, c_vp]),
     "gprb_lml_eval": (c_int, [c_vp, c_ll, c_int, c_int, c_vp, c_dbl, c_dbl, c_vp, c_ll, c_int, c_vp, c_int, c_int, c_int, c_int,
                              c_vp, c_vp, c_ll, c_vp, c_vp]),
     "gprb_chol_panel": (c_int, [c_vp, c_ll, c_int, c_int, c_int, c_vp, c_vp]),

@@ -2,7 +2,7 @@
 //
 // Replaces the scipy/numpy steps of GP.log_marginal_likelihood, GP.fit, GP.set_K_inv and
 // GP.predict* (gaussianprocess.py:128-202, 286-317, 338-377, 880-908).  The factorisation and
-// triangular solves are cuSOLVER (potrf / potrs / potri) and the K* K^-1 product is cuBLAS DGEMM:
+// triangular solves are cuSOLVER / cuBLAS (potrf / potrs / trsm) and the K* K^-1 product is cuBLAS trmm:
 // library calls, reported separately by bench.py and not optimised (north_star).  The
 // bandwidth-bound pieces (noise, log-det, trace of (alpha alpha^T - K^-1) dK, fused mean/variance
 // row reductions) are hand-written kernels with fixed-order reductions.
@@ -14,7 +14,6 @@
 #include <algorithm>
 #include <cusolverDn.h>
 #include <cublas_v2.h>
-#include <cstdlib>
 
 namespace {
 
@@ -66,7 +65,7 @@ struct Scratch {
 };
 
 // The Cholesky factor L lives in the row-major lower triangle == CUBLAS_FILL_MODE_UPPER of the column-major view the
-// libraries see (K = U^T U, U = L^T); every consumer below (potrs, trsm, potri) reads that triangle.  gprb_chol_factor
+// libraries see (K = U^T U, U = L^T); every consumer below (potrs, trsm) reads that triangle.  gprb_chol_factor
 // itself runs cuSOLVER's potrf in the OTHER fill mode, which is 20 % faster on B200 (357 vs 446 ms at N = 32 980,
 // profiles/r02_potrf_modes.txt), and mirrors the factor into the lower triangle afterwards (3 ms), so the trsm-heavy
 // consumers keep the mode in which cuBLAS trsm is faster (inverse rows: 990 vs 1 043 ms).
@@ -89,18 +88,6 @@ __global__ void mirror_upper_kernel(double *A, long long ld, int N) {
     __syncthreads();
     const int ti = bj * 32 + threadIdx.y, tj = bi * 32 + threadIdx.x;   // destination (transposed block)
     if (ti < N && tj < N && ti > tj) A[(long long)ti * ld + tj] = t[threadIdx.x][threadIdx.y];
-}
-
-// after potri on the (row-major) lower triangle: copy it to the upper triangle
-__global__ void mirror_lower_kernel(double *A, long long ld, int N) {
-    __shared__ double t[32][33];
-    const int bi = blockIdx.y, bj = blockIdx.x;
-    if (bj > bi) return;
-    const int i = bi * 32 + threadIdx.y, j = bj * 32 + threadIdx.x;
-    if (i < N && j < N) t[threadIdx.y][threadIdx.x] = A[(long long)i * ld + j];
-    __syncthreads();
-    const int ti = bj * 32 + threadIdx.y, tj = bi * 32 + threadIdx.x;   // transposed block
-    if (ti < N && tj < N && tj > ti) A[(long long)ti * ld + tj] = t[threadIdx.x][threadIdx.y];
 }
 
 __device__ __forceinline__ double block_sum(double v, double *sh) {
@@ -130,14 +117,14 @@ __global__ void lml_terms_kernel(const double *L, long long ld, int N, const dou
 // partial[3 b + 0] = sum over the block's rows of sum_j (alpha_i alpha_j - Kinv_ij) * dK_ij
 // partial[3 b + 1] = sum over rows of (alpha_i^2 - Kinv_ii) * w_i          (w = we / wf for energy / force rows)
 // partial[3 b + 2] = the same with the second weight pair (we2 / wf2)
-// KinvE != NULL (sharded inverse, gprb_lml_grad_trace_rows): the columns j < NE of a force row come from the
-// energy rows of the inverse, Kinv[i, j] = KinvE[j * ldE + i]; Kinv then only has to be valid for j >= i.
+// dK holds the rows of the row-sharded build: energy rows (i < NE) K_ee only, force rows K_fe and the J >= I blocks of
+// K_ff, so tr = EE (j in [i, NE), doubled off the diagonal) + 2 FE + FF (j >= i, doubled).  Kinv has to be valid for
+// j >= i only: the columns j < NE of a force row come from the energy rows of the inverse, Kinv[i, j] = KinvE[j * ldE + i].
 __global__ void __launch_bounds__(256) trace_kernel(int N, int r0, int r1, const double *__restrict__ alpha,
                                                     const double *__restrict__ Kinv, long long ldi,
                                                     const double *__restrict__ dK, long long lddk,
-                                                    int NE, double we, double wf, double we2, double wf2,
-                                                    int upper_only, double *partial,
-                                                    const double *__restrict__ KinvE = nullptr, long long ldE = 0) {
+                                                    int NE, double we, double wf, double we2, double wf2, double *partial,
+                                                    const double *__restrict__ KinvE, long long ldE) {
     __shared__ double sh[32];
     double acc = 0.0, acc2 = 0.0, acc3 = 0.0;
     for (int i = r0 + blockIdx.x; i < r1; i += gridDim.x) {
@@ -145,23 +132,13 @@ __global__ void __launch_bounds__(256) trace_kernel(int N, int r0, int r1, const
         const double *ki = Kinv + (long long)i * ldi;
         if (dK) {
             const double *di = dK + (long long)(i - r0) * lddk;
-            if (upper_only) {
-                // upper_only == 2 (row-sharded build): energy rows hold K_ee only, force rows hold K_fe and the
-                // J >= I blocks of K_ff:  tr = EE (upper, doubled) + 2 FE + FF (upper, doubled)
-                const int jend = (upper_only == 2 && i < NE) ? NE : N;
-                for (int j = i + threadIdx.x; j < jend; j += blockDim.x) {
-                    const double t = fma(ai, alpha[j], -ki[j]) * di[j];
-                    acc += (j == i) ? t : 2.0 * t;
-                }
-                if (upper_only == 2 && i >= NE) {
-                    if (KinvE)
-                        for (int j = threadIdx.x; j < NE; j += blockDim.x) acc += 2.0 * fma(ai, alpha[j], -KinvE[(long long)j * ldE + i]) * di[j];
-                    else
-                        for (int j = threadIdx.x; j < NE; j += blockDim.x) acc += 2.0 * fma(ai, alpha[j], -ki[j]) * di[j];
-                }
-            } else {
-                for (int j = threadIdx.x; j < N; j += blockDim.x) acc = fma(fma(ai, alpha[j], -ki[j]), di[j], acc);
+            const int jend = i < NE ? NE : N;
+            for (int j = i + threadIdx.x; j < jend; j += blockDim.x) {
+                const double t = fma(ai, alpha[j], -ki[j]) * di[j];
+                acc += (j == i) ? t : 2.0 * t;
             }
+            if (i >= NE)
+                for (int j = threadIdx.x; j < NE; j += blockDim.x) acc += 2.0 * fma(ai, alpha[j], -KinvE[(long long)j * ldE + i]) * di[j];
         }
         if (threadIdx.x == 0) {
             const double wii = ai * ai - ki[i];
@@ -186,51 +163,27 @@ __global__ void block_sum_kernel(int N, int r0, int r1, int c0, int c1, const do
     if (threadIdx.x == 0) { partial[3 * blockIdx.x] = acc; partial[3 * blockIdx.x + 1] = 0.0; partial[3 * blockIdx.x + 2] = 0.0; }
 }
 
-// out[k] (+)= 0.5 * sum_b partial[3 b + k]: one warp, lane-strided partial sums combined in a fixed order (deterministic)
-__global__ void final_sum_kernel(const double *partial, int n, double *out, int accumulate) {
+// out[k] += 0.5 * sum_b partial[3 b + k]: one warp, lane-strided partial sums combined in a fixed order (deterministic)
+__global__ void final_sum_kernel(const double *partial, int n, double *out) {
     double a = 0.0, b = 0.0, c = 0.0;
     for (int i = threadIdx.x; i < n; i += 32) { a += partial[3 * i]; b += partial[3 * i + 1]; c += partial[3 * i + 2]; }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         a += __shfl_xor_sync(0xffffffffu, a, o); b += __shfl_xor_sync(0xffffffffu, b, o); c += __shfl_xor_sync(0xffffffffu, c, o);
     }
-    if (threadIdx.x == 0) {
-        if (accumulate) { out[0] += 0.5 * a; out[1] += 0.5 * b; out[2] += 0.5 * c; }
-        else { out[0] = 0.5 * a; out[1] = 0.5 * b; out[2] = 0.5 * c; }
-    }
+    if (threadIdx.x == 0) { out[0] += 0.5 * a; out[1] += 0.5 * b; out[2] += 0.5 * c; }
 }
 
-// one CTA per test row: mean = Ks[i,:].alpha ; var = max(diag - Ks[i,:].W[i,:], 0)
+// one CTA per test row: mean = Ks[i,:].alpha
 __global__ void __launch_bounds__(256) predict_rows_kernel(int N, const double *__restrict__ Ks, long long ldks,
-                                                           const double *__restrict__ alpha, const double *__restrict__ W,
-                                                           const double *__restrict__ diag, double *mean, double *var) {
+                                                           const double *__restrict__ alpha, double *mean) {
     __shared__ double sh[32];
     const int i = blockIdx.x;
     const double *k = Ks + (long long)i * ldks;
-    double m = 0.0, v = 0.0;
-    if (W) {
-        const double *w = W + (long long)i * N;
-        for (int j = threadIdx.x; j < N; j += blockDim.x) { const double kj = k[j]; m = fma(kj, alpha[j], m); v = fma(kj, w[j], v); }
-    } else {
-        for (int j = threadIdx.x; j < N; j += blockDim.x) m = fma(k[j], alpha[j], m);
-    }
+    double m = 0.0;
+    for (int j = threadIdx.x; j < N; j += blockDim.x) m = fma(k[j], alpha[j], m);
     m = block_sum(m, sh);
-    v = block_sum(v, sh);
-    if (threadIdx.x == 0) {
-        mean[i] = m;
-        if (var) { const double r = diag[i] - v; var[i] = r < 0.0 ? 0.0 : r; }   // gaussianprocess.py:906-907
-    }
-}
-
-int copy_scalars(double *host, const double *dev, int n, cudaStream_t st) {
-    GPRB_CUDA(cudaMemcpyAsync(host, dev, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    GPRB_CUDA(cudaStreamSynchronize(st));
-    return GPRB_OK;
-}
-
-__global__ void set_identity_kernel(double *A, long long ld, int N) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < N) A[(long long)i * ld + i] = 1.0;
+    if (threadIdx.x == 0) mean[i] = m;
 }
 
 __global__ void unit_columns_kernel(double *B, long long ldb, int n_rows, int col0) {
@@ -238,7 +191,7 @@ __global__ void unit_columns_kernel(double *B, long long ldb, int n_rows, int co
     if (k < n_rows) B[(long long)k * ldb + col0 + k] = 1.0;
 }
 
-// ---- enqueue-only building blocks (no host synchronisation): shared by the granular entry points and gprb_lml_eval ----
+// ---- enqueue-only building blocks (no host synchronisation) of gprb_chol_factor, gprb_chol_inverse_rows and gprb_lml_eval ----
 
 // potrf in cuSOLVER's faster fill mode + mirror of the factor into the row-major lower triangle; *info_dev = potrf status
 int factor_enqueue(double *K, long long ldk, int N, int *info_dev, Scratch &scratch, cudaStream_t st) {
@@ -291,31 +244,31 @@ int inverse_rows_enqueue(const double *L, long long ldl, int N, int r0, int r1, 
 
 int trace_blocks(int rows) { return rows < 1184 ? rows : 1184; }     // 8 x 148
 
-// dev_out[0..2] (+)= {1/2 tr-term, 1/2 sum W_ii w_i, 1/2 sum W_ii w2_i} of the rows [r0, r1)
+// dev_out[0..2] += {1/2 tr-term, 1/2 sum W_ii w_i, 1/2 sum W_ii w2_i} of the rows [r0, r1)
 int trace_enqueue(int N, int r0, int r1, const double *alpha, const double *Kinv_virt, long long ldi, const double *dK_rows,
-                  long long lddk, int NE, double we, double wf, double we2, double wf2, int upper_only,
-                  const double *KinvE, long long ldE, double *dev_out, int accumulate, Scratch &scratch, cudaStream_t st) {
+                  long long lddk, int NE, double we, double wf, double we2, double wf2,
+                  const double *KinvE, long long ldE, double *dev_out, Scratch &scratch, cudaStream_t st) {
     const int blocks = trace_blocks(r1 - r0);
     double *d = (double *)scratch.get((size_t)3 * blocks * sizeof(double));
     if (!d) return GPRB_ERR_CUDA;
-    trace_kernel<<<blocks, 256, 0, st>>>(N, r0, r1, alpha, Kinv_virt, ldi, dK_rows, lddk, NE, we, wf, we2, wf2, upper_only, d, KinvE, ldE);
+    trace_kernel<<<blocks, 256, 0, st>>>(N, r0, r1, alpha, Kinv_virt, ldi, dK_rows, lddk, NE, we, wf, we2, wf2, d, KinvE, ldE);
     GPRB_LAUNCHED();
     GPRB_CUDA(cudaGetLastError());
-    final_sum_kernel<<<1, 32, 0, st>>>(d, blocks, dev_out, accumulate);
+    final_sum_kernel<<<1, 32, 0, st>>>(d, blocks, dev_out);
     GPRB_LAUNCHED();
     GPRB_CUDA(cudaGetLastError());
     return GPRB_OK;
 }
 
 int block_sum_enqueue(int N, int r0, int r1, int c0, int c1, const double *alpha, const double *Kinv, long long ldi,
-                      double *dev_out, int accumulate, Scratch &scratch, cudaStream_t st) {
+                      double *dev_out, Scratch &scratch, cudaStream_t st) {
     const int blocks = trace_blocks(r1 - r0);
     double *d = (double *)scratch.get((size_t)3 * blocks * sizeof(double));
     if (!d) return GPRB_ERR_CUDA;
     block_sum_kernel<<<blocks, 256, 0, st>>>(N, r0, r1, c0, c1, alpha, Kinv, ldi, d);
     GPRB_LAUNCHED();
     GPRB_CUDA(cudaGetLastError());
-    final_sum_kernel<<<1, 32, 0, st>>>(d, blocks, dev_out, accumulate);
+    final_sum_kernel<<<1, 32, 0, st>>>(d, blocks, dev_out);
     GPRB_LAUNCHED();
     GPRB_CUDA(cudaGetLastError());
     return GPRB_OK;
@@ -354,111 +307,6 @@ extern "C" int gprb_chol_factor(double *K, long long ldk, int N, void *stream) {
     return GPRB_OK;
 }
 
-extern "C" int gprb_chol_solve_vec(const double *L, long long ldl, int N, double *b, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(L && b && N > 0, "gprb_chol_solve_vec: bad argument");
-    int rc = handles(st);
-    if (rc) return rc;
-    Scratch scratch(st);
-    int *info = (int *)scratch.get(sizeof(int));
-    if (!info) return GPRB_ERR_CUDA;
-    return solve_vec_enqueue(L, ldl, N, b, info);
-}
-
-extern "C" int gprb_chol_inverse(const double *L, long long ldl, int N, double *Kinv, long long ldi, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(L && Kinv && N > 0, "gprb_chol_inverse: bad argument");
-    int rc = handles(st);
-    if (rc) return rc;
-    dim3 grid((N + 31) / 32, (N + 31) / 32), block(32, 32);
-    if ((long long)N * N >= (1LL << 31) || getenv("GPRB_FORCE_TRSM") != nullptr) {   // env: test hook for the large-N route
-        // cuSOLVER's potri (and the 64-bit trtri) reject N^2 >= 2^31 (N > 46340, e.g. the S4 configuration).
-        // Same result the way gaussianprocess.py:195 gets it, cho_solve(L, I): two triangular solves with
-        // the 64-bit cuBLAS interface on an identity right-hand side held in the output buffer.
-        GPRB_CUDA(cudaMemset2DAsync(Kinv, ldi * sizeof(double), 0, (size_t)N * sizeof(double), N, st));
-        set_identity_kernel<<<(N + 255) / 256, 256, 0, st>>>(Kinv, ldi, N);
-        GPRB_LAUNCHED();
-        const double one = 1.0;
-        // column-major view: K = U^T U with U in the upper triangle of L's buffer;  U^T Y = I, then U X = Y
-        cublasStatus_t b1 = cublasDtrsm_64(g_blas, CUBLAS_SIDE_LEFT, FACTOR_UPLO, solve_op(0), CUBLAS_DIAG_NON_UNIT,
-                                           (int64_t)N, (int64_t)N, &one, L, (int64_t)ldl, Kinv, (int64_t)ldi);
-        cublasStatus_t b2 = cublasDtrsm_64(g_blas, CUBLAS_SIDE_LEFT, FACTOR_UPLO, solve_op(1), CUBLAS_DIAG_NON_UNIT,
-                                           (int64_t)N, (int64_t)N, &one, L, (int64_t)ldl, Kinv, (int64_t)ldi);
-        if (b1 != CUBLAS_STATUS_SUCCESS || b2 != CUBLAS_STATUS_SUCCESS) {
-            gprb_set_error("cublasDtrsm_64 status %d / %d", (int)b1, (int)b2); return GPRB_ERR_CUDA;
-        }
-        mirror_lower_kernel<<<grid, block, 0, st>>>(Kinv, ldi, N);     // exactly symmetric, like the potri route
-        GPRB_LAUNCHED();
-        GPRB_CUDA(cudaGetLastError());
-        return GPRB_OK;
-    }
-    GPRB_CUDA(cudaMemcpy2DAsync(Kinv, ldi * sizeof(double), L, ldl * sizeof(double), (size_t)N * sizeof(double), N,
-                                cudaMemcpyDeviceToDevice, st));
-    int lwork = 0;
-    if (cusolverDnDpotri_bufferSize(g_solver, FACTOR_UPLO, N, Kinv, (int)ldi, &lwork) != CUSOLVER_STATUS_SUCCESS) {
-        gprb_set_error("potri_bufferSize failed"); return GPRB_ERR_CUDA;
-    }
-    Scratch scratch(st);
-    double *work = (double *)scratch.get((size_t)(lwork > 0 ? lwork : 1) * sizeof(double));
-    int *info = (int *)scratch.get(sizeof(int));
-    if (!work || !info) return GPRB_ERR_CUDA;
-    cusolverStatus_t cs = cusolverDnDpotri(g_solver, FACTOR_UPLO, N, Kinv, (int)ldi, work, lwork, info);
-    if (cs != CUSOLVER_STATUS_SUCCESS) { gprb_set_error("cusolverDnDpotri status %d", (int)cs); return GPRB_ERR_CUDA; }
-    mirror_lower_kernel<<<grid, block, 0, st>>>(Kinv, ldi, N);
-    GPRB_LAUNCHED();
-    GPRB_CUDA(cudaGetLastError());
-    return GPRB_OK;
-}
-
-extern "C" int gprb_lml_terms(const double *L, long long ldl, int N, const double *y, const double *alpha,
-                              double *out_host, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(L && y && alpha && out_host && N > 0, "gprb_lml_terms: bad argument");
-    { int rc0 = gprb_pool_init(); if (rc0) return rc0; }
-    Scratch scratch(st);
-    double *d = (double *)scratch.get(2 * sizeof(double));
-    if (!d) return GPRB_ERR_CUDA;
-    lml_terms_kernel<<<1, 1024, 0, st>>>(L, ldl, N, y, alpha, d);
-    GPRB_LAUNCHED();
-    GPRB_CUDA(cudaGetLastError());
-    return copy_scalars(out_host, d, 2, st);
-}
-
-extern "C" int gprb_lml_grad_trace(int N, int r0, int r1, const double *alpha, const double *Kinv, long long ldi,
-                                   const double *dK_rows, long long lddk, int NE, double we, double wf,
-                                   int upper_only, double *out_host, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(alpha && Kinv && out_host && 0 <= r0 && r0 <= r1 && r1 <= N, "gprb_lml_grad_trace: bad argument");
-    out_host[0] = out_host[1] = 0.0;
-    if (r0 == r1) return GPRB_OK;
-    { int rc0 = gprb_pool_init(); if (rc0) return rc0; }
-    Scratch scratch(st);
-    double *d = (double *)scratch.get(3 * sizeof(double));
-    if (!d) return GPRB_ERR_CUDA;
-    int rc = trace_enqueue(N, r0, r1, alpha, Kinv, ldi, dK_rows, lddk, NE, we, wf, 0.0, 0.0, upper_only, nullptr, 0, d, 0, scratch, st);
-    if (rc) return rc;
-    return copy_scalars(out_host, d, 2, st);
-}
-
-extern "C" int gprb_lml_grad_trace_rows(int N, int r0, int r1, const double *alpha, const double *Kinv_rows, long long ldr,
-                                        int c0, const double *KinvE, long long ldE, const double *dK_rows, long long lddk,
-                                        int NE, double we, double wf, double *out_host, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(alpha && Kinv_rows && out_host && 0 <= r0 && r0 <= r1 && r1 <= N && 0 <= c0 && c0 <= r0,
-                 "gprb_lml_grad_trace_rows: bad argument");
-    GPRB_REQUIRE(KinvE || r1 <= NE || NE == 0 || c0 == 0, "gprb_lml_grad_trace_rows: force rows need the energy rows of the inverse");
-    out_host[0] = out_host[1] = 0.0;
-    if (r0 == r1) return GPRB_OK;
-    { int rc0 = gprb_pool_init(); if (rc0) return rc0; }
-    Scratch scratch(st);
-    double *d = (double *)scratch.get(3 * sizeof(double));
-    if (!d) return GPRB_ERR_CUDA;
-    int rc = trace_enqueue(N, r0, r1, alpha, virtual_base(Kinv_rows, ldr, r0, c0), ldr, dK_rows, lddk, NE, we, wf, 0.0, 0.0, 2,
-                           KinvE, ldE, d, 0, scratch, st);
-    if (rc) return rc;
-    return copy_scalars(out_host, d, 2, st);
-}
-
 extern "C" int gprb_chol_inverse_rows(const double *L, long long ldl, int N, int r0, int r1, int c0,
                                       double *out, long long ldo, void *stream) {
     cudaStream_t st = (cudaStream_t)stream;
@@ -468,22 +316,6 @@ extern "C" int gprb_chol_inverse_rows(const double *L, long long ldl, int N, int
     int rc = handles(st);
     if (rc) return rc;
     return inverse_rows_enqueue(L, ldl, N, r0, r1, c0, out, ldo, st);
-}
-
-extern "C" int gprb_w_block_sum(int N, int r0, int r1, int c0, int c1, const double *alpha, const double *Kinv,
-                                long long ldi, double *out_host, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    GPRB_REQUIRE(alpha && Kinv && out_host && 0 <= r0 && r0 <= r1 && r1 <= N && 0 <= c0 && c0 <= c1 && c1 <= N,
-                 "gprb_w_block_sum: bad argument");
-    out_host[0] = 0.0;
-    if (r0 == r1 || c0 == c1) return GPRB_OK;
-    { int rc0 = gprb_pool_init(); if (rc0) return rc0; }
-    Scratch scratch(st);
-    double *d = (double *)scratch.get(3 * sizeof(double));
-    if (!d) return GPRB_ERR_CUDA;
-    int rc = block_sum_enqueue(N, r0, r1, c0, c1, alpha, Kinv, ldi, d, 0, scratch, st);
-    if (rc) return rc;
-    return copy_scalars(out_host, d, 1, st);
 }
 
 // One likelihood evaluation after the covariance build, enqueued back to back with ONE host synchronisation at the end
@@ -558,10 +390,10 @@ extern "C" int gprb_lml_eval(double *K, long long ldk, int N, int NE, const doub
                     rows = slab_buf;
                 }
                 const double *dptr = dK_rows ? dK_rows + (off + (a - R0)) * lddk : nullptr;
-                rc = trace_enqueue(N, a, b, alpha, virtual_base(rows, ldr, a, c0), ldr, dptr, lddk, NE, we, wf, we2, wf2, 2,
-                                   Einv, N, acc + 2, 1, scratch, st);
+                rc = trace_enqueue(N, a, b, alpha, virtual_base(rows, ldr, a, c0), ldr, dptr, lddk, NE, we, wf, we2, wf2,
+                                   Einv, N, acc + 2, scratch, st);
                 if (!rc && want_s0 && b <= NE)
-                    rc = block_sum_enqueue(N, a, b, 0, NE, alpha, Einv, N, acc + 5, 1, scratch, st);
+                    rc = block_sum_enqueue(N, a, b, 0, NE, alpha, Einv, N, acc + 5, scratch, st);
                 if (rc) return rc;
                 a = b;
             }
@@ -627,7 +459,7 @@ extern "C" int gprb_predict(int m, int N, const double *Ks, long long ldks, cons
     GPRB_REQUIRE(Ks && alpha && mean && m >= 0 && N > 0, "gprb_predict: bad argument");
     if (m == 0) return GPRB_OK;
     if (!var) {
-        predict_rows_kernel<<<m, 256, 0, st>>>(N, Ks, ldks, alpha, nullptr, diag, mean, var);
+        predict_rows_kernel<<<m, 256, 0, st>>>(N, Ks, ldks, alpha, mean);
         GPRB_LAUNCHED();
         GPRB_CUDA(cudaGetLastError());
         return GPRB_OK;

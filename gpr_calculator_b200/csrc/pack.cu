@@ -19,7 +19,7 @@ void gprb_set_error(const char *fmt, ...) {
 }
 
 extern "C" const char *gprb_last_error(void) { return g_err.c_str(); }
-extern "C" int gprb_version(void) { return 100; }
+extern "C" int gprb_version(void) { return 101; }
 
 std::atomic<long long> g_gprb_launches{0};
 extern "C" long long gprb_launch_count(void) { return g_gprb_launches.load(); }

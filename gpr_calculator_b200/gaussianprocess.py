@@ -5,9 +5,9 @@ methods, training-set containers, printed ``Loss:`` lines and guard behaviour.  
 where the arithmetic runs:
 
 * ``log_marginal_likelihood`` / ``fit`` (gaussianprocess.py:133-202, 222-317): K and dK/dl are
-  built on device by the kernel object, the noise is added, Cholesky / alpha / K^-1 come from
-  cuSOLVER (potrf / potrs / potri) and the gradient is the trace kernel of libgpr_b200 — K never
-  visits the host.  L-BFGS-B stays scipy on the host, as in the reference (:215-219).
+  built on device by the kernel object, the noise is added, Cholesky / alpha come from cuSOLVER
+  (potrf / potrs), the rows of K^-1 the gradient needs from triangular solves, and the gradient is
+  the trace kernel of libgpr_b200 — K never visits the host.  L-BFGS-B stays scipy on the host, as in the reference (:215-219).
 * ``predict`` / ``predict_structure`` (:319-379, 834-918): K* on device, mean and variance with
   the explicit K^-1 the reference uses (:128-131, 904-908), negative variances clipped to 0.
 * multi-GPU: with torch.distributed initialised (one process per GPU), each rank builds a row
@@ -334,18 +334,15 @@ class GP():
     def set_K_inv(self):
         """K^-1 = L^-T L^-1 (gaussianprocess.py:128-131) on device: blocks of rows right of the diagonal by
         trailing-block triangular solves written in place (gprb_chol_inverse_rows, the route of the likelihood
-        gradient: about 1.0 s instead of potri's 1.47 s at N = 32 980), then mirrored.  GPRB_FULL_INVERSE=1: potri."""
+        gradient: about 1.0 s instead of potri's 1.47 s at N = 32 980), then mirrored."""
         if self._Kinv_dev is None:
             N = self._L_dev.shape[0]
             Kinv = torch.empty((N, N), dtype=F64, device="cuda")
             st = stream()
-            if os.environ.get("GPRB_FULL_INVERSE", "0") not in ("", "0"):
-                _lib.call("gprb_chol_inverse", ptr(self._L_dev), N, N, ptr(Kinv), N, st)
-            else:
-                for (r0, r1, _) in _row_pieces([(0, N)], 0, N):
-                    _lib.call("gprb_chol_inverse_rows", ptr(self._L_dev), N, N, r0, r1, r0,
-                              c_vp(Kinv.data_ptr() + (r0 * N + r0) * 8), N, st)
-                _lib.call("gprb_symmetrize", ptr(Kinv), N, N, st)
+            for (r0, r1, _) in _row_pieces([(0, N)], 0, N):
+                _lib.call("gprb_chol_inverse_rows", ptr(self._L_dev), N, N, r0, r1, r0,
+                          c_vp(Kinv.data_ptr() + (r0 * N + r0) * 8), N, st)
+            _lib.call("gprb_symmetrize", ptr(Kinv), N, N, st)
             self._Kinv_dev = Kinv
 
     def log_marginal_likelihood(self, params, eval_gradient=False, clone_kernel=False):
@@ -368,12 +365,11 @@ class GP():
         K, dK, r_ranges = self._build_K(grad=eval_gradient)
         N = K.shape[0]
         NE = self._n_energy_rows()
-        full_inverse = os.environ.get("GPRB_FULL_INVERSE", "0") not in ("", "0")
-        if eval_gradient and is_rbf and not full_inverse and gdist.world()[1] > 1:
+        if eval_gradient and is_rbf and gdist.world()[1] > 1:
             dK, r_ranges = self._rebalance_dK(dK, r_ranges, N, NE)
         try:
-            alpha, out = self._lml_eval(K, dK if is_rbf else None, r_ranges, noise_e, noise_f,
-                                        want_grad=eval_gradient and not full_inverse, want_s0=not is_rbf)
+            _, out = self._lml_eval(K, dK if is_rbf else None, r_ranges, noise_e, noise_f,
+                                    want_grad=eval_gradient, want_s0=not is_rbf)
         except _lib.NotPositiveDefinite:
             return (-np.inf, np.zeros_like(params)) if eval_gradient else -np.inf
         logdet, ya = out[0], out[1]
@@ -387,11 +383,7 @@ class GP():
                 used = self._inverse_speed_used
                 self._inverse_speed = 0.5 * used / used.sum() + 0.5 * rates / rates.sum()
             self._inverse_cost = None
-        if full_inverse:
-            g_l, half_w_noise, half_w_base, g_s0 = self._lml_gradient_full_inverse(K, alpha, dK, r_ranges, N, NE, noise_e,
-                                                                                    noise_f, is_rbf)
-        else:
-            g_l, half_w_noise, half_w_base, g_s0 = out[2], out[3], out[4], out[5]
+        g_l, half_w_noise, half_w_base, g_s0 = out[2], out[3], out[4], out[5]
         if gdist.world()[1] > 1:
             g_l, half_w_noise, half_w_base, g_s0 = gdist.all_reduce_sum([g_l, half_w_noise, half_w_base, g_s0], device="cuda")
         if not is_rbf:
@@ -411,9 +403,9 @@ class GP():
         solves that follow cost (N - r)^2 per row, so the build's windows leave the first ranks with about twice the
         ideal solve time (SCALE_r01: 221 ms on rank 0 at 8 GPUs against 124 ms ideal).  dK/dl is only consumed by the
         traces, so its force rows are exchanged (one all-to-all over NVLink, about a third of the slab) into windows
-        balanced for the solves; K is untouched.  GPRB_BALANCE_INVERSE=0 keeps the build's windows."""
+        balanced for the solves; K is untouched."""
         rank, size = gdist.world()
-        if os.environ.get("GPRB_BALANCE_INVERSE", "1") in ("", "0") or dK is None or len(r_ranges) != 2:
+        if dK is None or len(r_ranges) != 2:
             return dK, r_ranges
         (e0, e1), (r0, r1) = r_ranges
         NF = (N - NE) // 3
@@ -488,40 +480,6 @@ class GP():
                   ptr(dK), dK.stride(0) if dK is not None else N, len(r_ranges), ranges, int(bool(want_grad)),
                   int(bool(want_s0)), parts, prefactored, ptr(alpha), ptr(work), n_work, out, stream())
         return alpha, [float(v) for v in out]
-
-    def _lml_gradient_full_inverse(self, K, alpha, dK, r_ranges, N, NE, noise_e, noise_f, is_rbf):
-        """The reference's literal route (gaussianprocess.py:195): the explicit inverse on every rank (cuSOLVER potri),
-        kept behind GPRB_FULL_INVERSE=1 as the cross-check of the inverse-rows route."""
-        st = stream()
-        out = (ctypes_double * 2)()
-        sharded = gdist.world()[1] > 1
-        Kinv = torch.empty((N, N), dtype=F64, device="cuda")
-        _lib.call("gprb_chol_inverse", ptr(K), N, N, ptr(Kinv), N, st)
-        # 1/2 tr(W dK/dl) over the rows of dK held by this rank (W, dK symmetric: columns j >= i,
-        # off-diagonal terms doubled -- the blocks left of the diagonal are not built when sharded)
-        # + 1/2 sum_i W_ii noise_i^2 (for the sigma term)
-        g_l = half_w_noise = half_w_base = g_s0 = 0.0
-        off = 0
-        for (r0, r1) in r_ranges:
-            if r1 > r0:
-                dptr = c_vp(0)
-                if is_rbf:
-                    dptr = c_vp(dK.data_ptr() + off * dK.stride(0) * 8)
-                _lib.call("gprb_lml_grad_trace", N, r0, r1, ptr(alpha), ptr(Kinv), N, dptr, dK.stride(0) if is_rbf else N, NE,
-                          float(noise_e) ** 2, float(noise_f) ** 2, 2 if sharded else 1, out, st)
-                g_l += out[0]
-                half_w_noise += out[1]
-                _lib.call("gprb_lml_grad_trace", N, r0, r1, ptr(alpha), ptr(Kinv), N, c_vp(0), N, NE,
-                          2.0 * float(noise_e), 2.0 * float(noise_f), 1, out, st)
-                half_w_base += out[1]
-            off += r1 - r0
-        if not is_rbf:
-            (r0, r1) = r_ranges[0]
-            r1 = min(r1, NE)            # energy rows held by this rank (the first range starts with them)
-            if r1 > r0 and NE > 0:
-                _lib.call("gprb_w_block_sum", N, r0, r1, 0, NE, ptr(alpha), ptr(Kinv), N, out, st)
-                g_s0 = out[0]
-        return g_l, half_w_noise, half_w_base, g_s0
 
     def optimize(self, fun, theta0, bounds, maxiter=10):
         """L-BFGS-B on the host, identical options to gaussianprocess.py:215-219."""

@@ -140,60 +140,32 @@ int gprb_add_noise(double *K_dev, long long ldk, int N, int NE, double noise_e, 
 /* In-place Cholesky K = L L^T (cuSOLVER potrf).  Returns GPRB_ERR_LINALG if not positive definite
  * (the reference maps that to LML = -inf, gaussianprocess.py:174-177). */
 int gprb_chol_factor(double *K_dev, long long ldk, int N, void *stream);
-/* Solve (L L^T) X = B in place for nrhs right-hand sides stored as columns of a row-major
- * [N, nrhs] matrix when nrhs == 1, i.e. a plain vector (cuSOLVER potrs). */
-int gprb_chol_solve_vec(const double *L_dev, long long ldl, int N, double *b_dev, void *stream);
-/* Kinv = (L L^T)^-1, full symmetric matrix, out of place (cuSOLVER potri + mirror)
- * (gaussianprocess.py:128-131, 195). */
-int gprb_chol_inverse(const double *L_dev, long long ldl, int N, double *Kinv_dev, long long ldi, void *stream);
 /* A[i][j] = A[j][i] for all i > j of the n x n block at A (fills the lower triangle from the upper
  * one after an all-gather of GPRB_FF_UPPER row blocks). */
 int gprb_symmetrize(double *A_dev, long long ld, int n, void *stream);
 /* dst[j*ldd + i] = src[i*lds + j] for a rows x cols block (K_ef = K_fe^T after a row-sharded build). */
 int gprb_transpose_copy(double *dst_dev, long long ldd, const double *src_dev, long long lds, int rows, int cols, void *stream);
-/* out_host[0] = sum_i log L_ii ; out_host[1] = y.alpha                 (gaussianprocess.py:183-186) */
-int gprb_lml_terms(const double *L_dev, long long ldl, int N, const double *y_dev, const double *alpha_dev,
-                   double *out_host, void *stream);
-/* out_host[0] = 1/2 sum_{i in [r0,r1), j} (alpha_i alpha_j - Kinv_ij) dK_ij  with dK given for
- * rows [r0,r1) only (row-block sharded; all-reduce the scalar across ranks).
- * out_host[1] = 1/2 sum_i (alpha_i^2 - Kinv_ii) * w_i, w_i = (i<NE ? we : wf) over the same rows
- * (noise / sigma terms).                                           (gaussianprocess.py:188-198)
- * upper_only = 1: dK holds valid entries only for columns j >= i (GPRB_FF_UPPER build); the sum
- * then runs over j >= i with weight 2 off the diagonal (W and dK are symmetric).
- * upper_only = 2: row-sharded build: energy rows (i < NE) hold dK_ee only, force rows hold dK_fe and
- * the J >= I blocks of dK_ff: sum = EE (j in [i, NE), doubled) + 2 FE + FF (j >= i, doubled). */
-int gprb_lml_grad_trace(int N, int r0, int r1, const double *alpha_dev, const double *Kinv_dev, long long ldi,
-                        const double *dK_rows_dev, long long lddk, int NE, double we, double wf,
-                        int upper_only, double *out_host, void *stream);
 /* Rows of the inverse without forming it (row-sharded likelihood gradient: a rank that holds the rows
  * [r0, r1) of dK with valid entries right of the diagonal only needs Kinv[r0:r1, c0:N] with c0 <= r0):
  *   out[k*ldo + t] = Kinv[r0 + k, c0 + t],  k < r1 - r0,  t < N - c0,
  * from the TRAILING block of the factor, K^-1[T,T] = (L_TT L_TT^T)^-1 for T = [c0, N) (two cuBLAS trsm, i.e. potrs, with
  * r1 - r0 unit right-hand sides on the (N - c0)-dimensional trailing system: 2 (N-c0)^2 (r1-r0) flops
- * instead of the 2 N^3 / 3 of potri on every rank).  c0 = 0 gives full rows (the energy rows). */
+ * instead of forming the whole inverse on every rank).  c0 = 0 gives full rows (the energy rows). */
 int gprb_chol_inverse_rows(const double *L_dev, long long ldl, int N, int r0, int r1, int c0,
                            double *out_dev, long long ldo, void *stream);
-/* gprb_lml_grad_trace(upper_only = 2) on such slabs: Kinv_rows_dev = the slab of rows [r0, r1) from
- * gprb_chol_inverse_rows(..., c0, ...) with leading dimension ldr; KinvE_dev = Kinv[0:NE, :] ([NE, ldE]
- * row-major, from gprb_chol_inverse_rows(0, NE, 0)) supplies the columns j < NE of force rows
- * (may be NULL when r1 <= NE or NE == 0). */
-int gprb_lml_grad_trace_rows(int N, int r0, int r1, const double *alpha_dev, const double *Kinv_rows_dev, long long ldr,
-                             int c0, const double *KinvE_dev, long long ldE, const double *dK_rows_dev, long long lddk,
-                             int NE, double we, double wf, double *out_host, void *stream);
 /* Live FP64 tensor-pipe roofline denominator: DMMA.8x8x4 issue-rate micro-benchmark (all SMs,
  * 16 independent accumulators per warp).  MEASURED_PEAKS.json carries no fp64 entry. */
 int gprb_fp64_dmma_peak(double *tflops_host, void *stream);
-/* 1/2 sum over the block [r0,r1) x [c0,c1) of (alpha_i alpha_j - Kinv_ij)   (Dot d/dsigma0 term) */
-int gprb_w_block_sum(int N, int r0, int r1, int c0, int c1, const double *alpha_dev, const double *Kinv_dev,
-                     long long ldi, double *out_host, void *stream);
 /* One likelihood evaluation after the covariance build, enqueued back to back with a single host synchronisation
  * (GP.log_marginal_likelihood, gaussianprocess.py:160-198; the scipy cholesky / cho_solve / einsum steps of :174-198):
  * K += noise on the diagonal, in-place Cholesky, alpha = K^-1 y, and -- want_grad -- the traces of
  * W = alpha alpha^T - K^-1 against the rows of dK/dl this rank holds, K^-1 taken block of rows by block of rows
  * (N / parts rows, >= 512) from trailing-block triangular solves as in gprb_chol_inverse_rows (no explicit inverse).
  *   ranges_host[2 n_ranges]: row ranges (r0, r1) of the assembled matrix whose rows of dK are stacked in
- *     dK_rows_dev (leading dimension lddk; NULL = no dK term); rows < NE carry the K_ee part, force rows K_fe and
- *     the J >= I blocks of K_ff (the layout of gprb_lml_grad_trace with upper_only = 2; a full dK satisfies it).
+ *     dK_rows_dev (leading dimension lddk; NULL = no dK term).  Only the entries of the row-sharded build are read:
+ *     an energy row i < NE reads the K_ee columns j in [i, NE), a force row i >= NE the K_fe columns j < NE and the
+ *     columns j >= i (J >= I blocks of K_ff); W and dK are symmetric, so off-diagonal terms count twice.  A full dK
+ *     satisfies this layout.
  *   alpha_dev[N] receives alpha; K_dev holds the factor on return.
  *   out_host[8]: [0] sum_i log L_ii, [1] y.alpha, [2] 1/2 tr(W dK) over the held rows, [3] 1/2 sum W_ii noise_i^2,
  *     [4] 1/2 sum W_ii 2 noise_i, [5] 1/2 sum of W over (held energy rows) x (all energy columns) when want_s0

@@ -152,22 +152,30 @@ def add_noise(K, NE, noise_e, noise_f):
     return K
 
 
+def lml_from_matrices(K, dK, y_train, NE, noise_e, noise_f):
+    """The algebra of gaussianprocess.py:162-198 on given matrices: K is the noise-free covariance [N, N] (the first NE
+    rows are energy rows), dK[:, :, k] = dK/dtheta_k (None: no gradient), y_train [N] or [N, 1].
+    Returns the LML, or (LML, gradient) when dK is given."""
+    y_train = np.asarray(y_train, dtype=np.float64).reshape(len(K), -1)
+    K = add_noise(K, NE, noise_e, noise_f)
+    L = cholesky(K, lower=True)
+    alpha = cho_solve((L, True), y_train)
+    mll = -0.5 * float(y_train[:, 0] @ alpha[:, 0]) - np.log(np.diag(L)).sum() - len(K) / 2 * np.log(2 * np.pi)
+    if dK is None:
+        return mll
+    W = alpha @ alpha.T - cho_solve((L, True), np.eye(len(K)))
+    grad = 0.5 * np.einsum("ij,jik->k", W, dK)
+    return mll, grad
+
+
 def log_marginal_likelihood(kernel, train_x, y_train, noise_e, noise_f, eval_gradient=True):
     """gaussianprocess.py:160-202 with fixed noise (noise_bounds is None)."""
     NE = len(train_x["energy"][-1]) if len(train_x["energy"]) > 0 else 0
     if eval_gradient:
         K, dK = kernel.k_total_with_grad(train_x)
     else:
-        K = kernel.k_total(train_x)
-    K = add_noise(K, NE, noise_e, noise_f)
-    L = cholesky(K, lower=True)
-    alpha = cho_solve((L, True), y_train)
-    mll = -0.5 * float(y_train[:, 0] @ alpha[:, 0]) - np.log(np.diag(L)).sum() - len(K) / 2 * np.log(2 * np.pi)
-    if not eval_gradient:
-        return mll
-    W = alpha @ alpha.T - cho_solve((L, True), np.eye(len(K)))
-    grad = 0.5 * np.einsum("ij,jik->k", W, dK)
-    return mll, grad
+        K, dK = kernel.k_total(train_x), None
+    return lml_from_matrices(K, dK, y_train, NE, noise_e, noise_f)
 
 
 def fit_factors(kernel, train_x, y_train, noise_e, noise_f):

@@ -1,6 +1,7 @@
 """Worker of tests/test_gpu_multi.py (run under torchrun, one rank per GPU): the row-sharded covariance build
 with the gather fused into the kernels (NVLink peer stores) against the NCCL all-gather build and the
-single-GPU build of the same training set, then LML + gradient through both sharded paths."""
+single-GPU build of the same training set, then LML + gradient through the sharded paths against the reference's
+algebra evaluated on the host (oracle.gp.lml_from_matrices) on the unsharded K and dK/dl."""
 import os
 import sys
 
@@ -22,6 +23,7 @@ def main():
     from gpr_calculator_b200.SO3 import SO3
     from gpr_calculator_b200.gaussianprocess import GP
     from gpr_calculator_b200.kernels import RBF_mb
+    from oracle import gp as ogp
 
     labelled = syn.structures(n_struct, 2, 2000)
     des = SO3(nmax=3, lmax=4, rcut=5.0)
@@ -43,11 +45,13 @@ def main():
     gp0 = make_gp()
     K1, dK1 = gp0.kernel.k_total_device(gp0.train_x, None, f_tol=1e-10, grad=True)
     scale = float(K1.abs().max())
+    NE = e_pack.n_groups
+    K1h = K1.cpu().numpy()
+    lml_h, g_h = ogp.lml_from_matrices(K1h, np.dstack((2 * K1h / theta[0], dK1.cpu().numpy())), y, NE, 0.002, 0.1)
 
     results = {}
-    for mode in ("peer", "nccl", "fullinv", "distchol"):
+    for mode in ("peer", "nccl", "distchol"):
         os.environ["GPRB_NO_PEER"] = "1" if mode == "nccl" else "0"
-        os.environ["GPRB_FULL_INVERSE"] = "1" if mode == "fullinv" else "0"     # potri on every rank instead of inverse rows
         # "distchol": the factorisation shared by the ranks (dist.distributed_cholesky, panels of 256 rows) instead of repeated on each
         GP.DIST_CHOLESKY_MIN_N = 512 if mode == "distchol" else 10 ** 9
         os.environ["GPRB_DIST_CHOLESKY_NB"] = "256"
@@ -61,7 +65,6 @@ def main():
             assert getattr(gp, "_peer", None) is None
         err = float((K - K1).abs().max()) / scale
         # dK rows held by this rank (energy rows: K_ee part only; force rows: K_fe and the J >= I blocks)
-        NE = e_pack.n_groups
         off, derr = 0, 0.0
         for (r0, r1) in ranges:
             rows = dK[off:off + (r1 - r0)]
@@ -88,27 +91,23 @@ def main():
     same = float((Kp - Kn).abs().max()) <= 1e-13 * scale
     lml_p, g_p = results["peer"][3], results["peer"][4]
     lml_n, g_n = results["nccl"][3], results["nccl"][4]
-    # single-GPU LML on rank-local unsharded algebra: same GP code with world pretending 1 is not possible
-    # inside a process group, so compare the two sharded paths with each other and K with the unsharded build
-    lml_f, g_f = results["fullinv"][3], results["fullinv"][4]
     lml_d, g_d = results["distchol"][3], results["distchol"][4]
     GP.DIST_CHOLESKY_MIN_N = 512          # the fit / prediction checks below run on the shared factorisation too
-    # Dot kernel: the d/dsigma0 term of the sharded gradient against the potri route
+    # Dot kernel: the d/dsigma0 term of the sharded gradient (E-E constant of dot_kernel.py:58) against the host
     from gpr_calculator_b200.kernels import Dot_mb
-    dot = {}
-    for mode in ("rows", "fullinv"):
-        os.environ["GPRB_FULL_INVERSE"] = "1" if mode == "fullinv" else "0"
-        gd_ = GP(kernel=Dot_mb(para=[2.0, 1.5], zeta=3), descriptor=des, noise_e=0.002, noise_f=0.1, log_file=None)
-        gd_.train_x = {"energy": e_pack, "force": f_pack}
-        gd_.y_train = y
-        dot[mode] = gd_.log_marginal_likelihood(np.array([2.0, 1.5]), eval_gradient=True)
-        gd_.release_peer()
-    dot_ok = (abs(dot["rows"][0] - dot["fullinv"][0]) <= 1e-9 * abs(dot["fullinv"][0])
-              and np.allclose(dot["rows"][1], dot["fullinv"][1], rtol=1e-7, atol=1e-7))
+    gd_ = GP(kernel=Dot_mb(para=[2.0, 1.5], zeta=3), descriptor=des, noise_e=0.002, noise_f=0.1, log_file=None)
+    gd_.train_x = {"energy": e_pack, "force": f_pack}
+    gd_.y_train = y
+    dot = gd_.log_marginal_likelihood(np.array([2.0, 1.5]), eval_gradient=True)
+    gd_.release_peer()
+    Kd = gd_.kernel.k_total_device(gd_.train_x, None, grad=True)[0].cpu().numpy()
+    Cs0 = np.zeros_like(Kd)
+    Cs0[:NE, :NE] = 0.8 * 2 * 2.0 ** 2 * 1.5
+    dot_h = ogp.lml_from_matrices(Kd, np.dstack((2 * Kd / 2.0, Cs0)), y, NE, 0.002, 0.1)
+    dot_ok = abs(dot[0] - dot_h[0]) <= 1e-9 * abs(dot_h[0]) and np.allclose(dot[1], dot_h[1], rtol=1e-7, atol=1e-7)
     # sharded prediction (structures split over the ranks, results all-reduced) against every rank predicting everything,
     # and a full fit with the optimiser values broadcast from rank 0: identical hyper-parameters on every rank
     os.environ["GPRB_NO_PEER"] = "0"
-    os.environ["GPRB_FULL_INVERSE"] = "0"
     gpp = make_gp()
     gpp.fit(opt=True, show=False, maxiter=3)
     theta_fit = torch.tensor(gpp.kernel.parameters(), dtype=torch.float64, device="cuda")
@@ -128,11 +127,11 @@ def main():
               % (pred_err, same_theta, gpp.kernel.parameters()), flush=True)
     ok = (pred_ok and results["peer"][1] <= 1e-12 and results["nccl"][1] <= 1e-12 and results["peer"][2] <= 1e-12 and same
           and abs(lml_p - lml_n) <= 1e-9 * abs(lml_n) and np.allclose(g_p, g_n, rtol=1e-9, atol=1e-9)
-          and abs(lml_p - lml_f) <= 1e-9 * abs(lml_f) and np.allclose(g_p, g_f, rtol=1e-7, atol=1e-7) and dot_ok
+          and abs(lml_p - lml_h) <= 1e-9 * abs(lml_h) and np.allclose(g_p, g_h, rtol=1e-7, atol=1e-7) and dot_ok
           and abs(lml_p - lml_d) <= 1e-10 * abs(lml_p) and np.allclose(g_p, g_d, rtol=1e-8, atol=1e-8))
     if rank == 0:
-        print("gradient rows %s | potri %s | shared Cholesky %s (lml %.12g vs %.12g); Dot rows %s | potri %s"
-              % (g_p, g_f, g_d, lml_d, lml_p, dot["rows"], dot["fullinv"]), flush=True)
+        print("gradient rows %s | host %s | shared Cholesky %s (lml %.12g vs %.12g, host %.12g); Dot rows %s | host %s"
+              % (g_p, g_h, g_d, lml_d, lml_p, lml_h, dot, dot_h), flush=True)
     flag = torch.tensor([1 if ok else 0], device="cuda")
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     print("[rank %d/%d] N=%d K err peer %.2e nccl %.2e dK err %.2e bitwise(peer,nccl)=%s lml %.9f / %.9f grad %s / %s"

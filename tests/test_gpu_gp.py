@@ -187,33 +187,33 @@ def test_gpr_calculator_adapter(capsys):
     assert gp.use_base == n_base             # frozen: the base calculator is not called
 
 
-def test_inverse_large_n_route_matches_potri(monkeypatch):
-    """gprb_chol_inverse switches from potri to two 64-bit triangular solves when N^2 >= 2^31 (S4: N = 65000); the test hook
-    forces that route at a small size and compares both against numpy."""
-    import torch
-    from gpr_calculator_b200 import _lib
-    from gpr_calculator_b200.device import ptr, stream
-    rng = np.random.default_rng(3)
-    N = 300
-    A = rng.normal(size=(N, N))
-    K = A @ A.T + N * np.eye(N)
-    Kd = torch.as_tensor(K, device="cuda").contiguous()
-    _lib.call("gprb_chol_factor", ptr(Kd), N, N, stream())
-    outs = []
-    for force in (False, True):
-        if force:
-            monkeypatch.setenv("GPRB_FORCE_TRSM", "1")
-        Kinv = torch.empty((N, N), dtype=torch.float64, device="cuda")
-        _lib.call("gprb_chol_inverse", ptr(Kd), N, N, ptr(Kinv), N, stream())
-        outs.append(Kinv.cpu().numpy())
-    ref = np.linalg.inv(K)
-    for o in outs:
-        assert rel_err(o, ref) <= 1e-10 and np.abs(o - o.T).max() == 0.0
+def _oracle_lml(gp, theta):
+    """oracle.gp.lml_from_matrices on the noise-free K (and dK/dl) the GP builds on device, with the gradient components of
+    GP.log_marginal_likelihood: 2K/sigma, then dK/dl (RBF) or the E-E constant d/dsigma0 of dot_kernel.py:58 (Dot), then
+    diag(2 noise_i) when the noise is a hyper-parameter (gaussianprocess.py:196-198)."""
+    from oracle import gp as ogp
+    ker = gp.kernel
+    ker.update(theta if gp.noise_bounds is None else theta[:-1])
+    Kd, dKd = ker.k_total_device(gp.train_x, None, f_tol=1e-10, grad=True)
+    K = Kd.cpu().numpy()
+    NE = gp._n_energy_rows()
+    if dKd is not None:
+        dK = dKd.cpu().numpy()
+    else:
+        dK = np.zeros_like(K)
+        dK[:NE, :NE] = 0.8 * 2 * ker.sigma ** 2 * ker.sigma0
+    comps = [2 * K / ker.sigma, dK]
+    noise_e, noise_f = gp.noise_e, gp.noise_f
+    if gp.noise_bounds is not None:
+        noise_e, noise_f = theta[-1], gp.f_coef * theta[-1]
+        comps.append(np.diag(np.where(np.arange(len(K)) < NE, 2 * noise_e, 2 * noise_f)))
+    return ogp.lml_from_matrices(K, np.dstack(comps), gp.y_train, NE, noise_e, noise_f)
 
 
-def test_inverse_rows_and_gradient_routes(g, monkeypatch):
-    """gprb_chol_inverse_rows against numpy (trailing-block solves), and the likelihood gradient through the blocked
-    inverse-rows route against the literal route of the reference (explicit inverse, gaussianprocess.py:195)."""
+def test_inverse_rows_and_gradient_routes(g):
+    """gprb_chol_inverse_rows against numpy (trailing-block solves), and the likelihood and its gradient (blocked
+    inverse-rows route of gprb_lml_eval) against the reference's algebra evaluated on the host on the same K and dK
+    (explicit inverse, gaussianprocess.py:195)."""
     import torch
     from gpr_calculator_b200 import _lib
     from gpr_calculator_b200.device import ptr, stream
@@ -230,23 +230,29 @@ def test_inverse_rows_and_gradient_routes(g, monkeypatch):
         if r1 > r0:
             assert rel_err(out[:, :N - c0].cpu().numpy(), ref[r0:r1, c0:]) <= 1e-10
             assert bool((out[:, N - c0:] == 7.0).all())
-    for kernel, theta in (("RBF", np.array([1.3, 0.25])), ("Dot", np.array([2.0, 1.5]))):
+    cases = [("RBF", np.array([1.3, 0.25]), None), ("Dot", np.array([2.0, 1.5]), None),
+             # a noise hyper-parameter adds the third gradient component (noise_bounds, gaussianprocess.py:196-198)
+             ("RBF", np.array([1.3, 0.25, 0.004]), [1e-4, 1e-1])]
+    for kernel, theta, noise_bounds in cases:
         gp = _model(g, kernel)
-        monkeypatch.setenv("GPRB_FULL_INVERSE", "0")
-        lml_r, grad_r = gp.log_marginal_likelihood(theta, eval_gradient=True)
-        monkeypatch.setenv("GPRB_FULL_INVERSE", "1")
-        lml_f, grad_f = gp.log_marginal_likelihood(theta, eval_gradient=True)
-        assert lml_r == lml_f
-        assert np.allclose(grad_r, grad_f, rtol=1e-9, atol=1e-9 * max(1.0, np.abs(grad_f).max()))
-    # a noise hyper-parameter adds the third gradient component (noise_bounds, gaussianprocess.py:196-198)
-    gp = _model(g, "RBF")
-    gp.noise_bounds = [1e-4, 1e-1]
-    th = np.array([1.3, 0.25, 0.004])
-    monkeypatch.setenv("GPRB_FULL_INVERSE", "0")
-    _, grad_r = gp.log_marginal_likelihood(th, eval_gradient=True)
-    monkeypatch.setenv("GPRB_FULL_INVERSE", "1")
-    _, grad_f = gp.log_marginal_likelihood(th, eval_gradient=True)
-    assert len(grad_r) == 3 and np.allclose(grad_r, grad_f, rtol=1e-9, atol=1e-9 * np.abs(grad_f).max())
+        gp.noise_bounds = noise_bounds
+        lml, grad = gp.log_marginal_likelihood(theta, eval_gradient=True)
+        lml_h, grad_h = _oracle_lml(gp, theta)
+        assert len(grad) == len(theta)
+        assert abs(lml - lml_h) <= 1e-12 * abs(lml_h), (kernel, lml, lml_h)
+        assert np.allclose(grad, grad_h, rtol=1e-9, atol=1e-9 * np.abs(grad_h).max()), (kernel, grad, grad_h)
+
+
+def _inverse_as_set_K_inv(Ld, N):
+    """K^-1 from the factor the way GP.set_K_inv forms it: rows right of the diagonal by trailing-block solves, then mirrored."""
+    import torch
+    from gpr_calculator_b200 import _lib
+    from gpr_calculator_b200.device import c_vp, ptr, stream
+    Kinv = torch.empty((N, N), dtype=torch.float64, device="cuda")
+    for r0, r1 in ((0, N // 3), (N // 3, N)):
+        _lib.call("gprb_chol_inverse_rows", ptr(Ld), N, N, r0, r1, r0, c_vp(Kinv.data_ptr() + (r0 * N + r0) * 8), N, stream())
+    _lib.call("gprb_symmetrize", ptr(Kinv), N, N, stream())
+    return Kinv
 
 
 def test_variance_routes_match_numpy(g, monkeypatch):
@@ -266,8 +272,7 @@ def test_variance_routes_match_numpy(g, monkeypatch):
     want_var = np.maximum(prior - quad, 0.0)
     Ld = torch.as_tensor(K, device="cuda").contiguous()
     _lib.call("gprb_chol_factor", ptr(Ld), N, N, stream())
-    Kinv = torch.empty((N, N), dtype=torch.float64, device="cuda")
-    _lib.call("gprb_chol_inverse", ptr(Ld), N, N, ptr(Kinv), N, stream())
+    Kinv = _inverse_as_set_K_inv(Ld, N)
     Kd = torch.as_tensor(np.ascontiguousarray(rng.normal(size=(m, N + 5))), device="cuda")
     Kd[:, :N] = torch.as_tensor(Ks, device="cuda")
     ad, dd = torch.as_tensor(alpha, device="cuda"), torch.as_tensor(prior, device="cuda")

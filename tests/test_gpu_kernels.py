@@ -189,18 +189,58 @@ def test_modes_and_windows_agree():
         assert (Kf - 1.3 ** 2 * K1).abs().max().item() <= 1e-13 * scale
 
 
-def test_upper_mode_windows_symmetrize_and_trace():
-    """The sharded build: every rank writes the J >= I blocks of its row window (FF_UPPER) into the full
-    matrix, gprb_symmetrize mirrors them; the upper-only gradient trace equals the full one."""
+def _lml_eval(K, dK_rows, ranges, NE, y, noise_e, noise_f):
+    """gprb_lml_eval with the gradient traces on a copy of K (noise and factor are applied in place): out[0..5]."""
     import ctypes
+    from gpr_calculator_b200 import _lib
+    from gpr_calculator_b200.device import ptr, stream
+    N = K.shape[0]
+    Kc = K.clone()
+    alpha = torch.empty(N, dtype=torch.float64, device="cuda")
+    n_work = int(_lib.load().gprb_lml_eval_work(N, NE, 1, 16))
+    work = torch.empty(n_work, dtype=torch.float64, device="cuda")
+    flat = [v for r in ranges for v in r]
+    out = (ctypes.c_double * 8)()
+    _lib.call("gprb_lml_eval", ptr(Kc), N, N, NE, ptr(y), float(noise_e), float(noise_f), ptr(dK_rows), dK_rows.stride(0),
+              len(ranges), (ctypes.c_int * len(flat))(*flat), 1, 0, 16, 0, ptr(alpha), ptr(work), n_work, out, stream())
+    return np.array(out[:6])
+
+
+def _trace_vs_oracle(K, dK, NE, y, noise_e, noise_f, out):
+    """out[2..4] of gprb_lml_eval (1/2 tr(W dK), 1/2 sum W_ii noise_i^2, 1/2 sum W_ii 2 noise_i) against the reference's
+    algebra on the host (oracle.gp.lml_from_matrices), K + noise kept at cond <= 1e6.  Returns error / tolerance."""
+    from oracle import gp as ogp
+    Kh, dKh = K.cpu().numpy(), dK.cpu().numpy()
+    noise = np.where(np.arange(len(Kh)) < NE, noise_e, noise_f)
+    assert np.linalg.cond(Kh + np.diag(noise ** 2)) <= 1e6
+    _, want = ogp.lml_from_matrices(Kh, np.dstack((dKh, np.diag(noise ** 2), np.diag(2 * noise))), y.cpu().numpy(), NE,
+                                    noise_e, noise_f)
+    ratio = np.abs(out[2:5] - want) / (1e-9 * np.abs(want) + 1e-9 * np.abs(want).max())
+    assert ratio.max() <= 1.0, (out[2:5], want)
+    return ratio.max()
+
+
+def test_upper_mode_windows_symmetrize_and_trace(capsys):
+    """The sharded build: every rank writes the J >= I blocks of its row window (FF_UPPER) into the full
+    matrix, gprb_symmetrize mirrors them; the likelihood traces of gprb_lml_eval read dK right of the diagonal only."""
     from gpr_calculator_b200 import _lib, dist as gd
-    from gpr_calculator_b200.device import Pack, k_total_device, build_force_rows, ptr, stream, c_vp
+    from gpr_calculator_b200.device import Pack, k_total_device, build_force_rows, ptr, stream
     from gpr_calculator_b200.utilities import list_to_tuple
     rng = np.random.default_rng(11)
     X, dX, ELE, ind = list_to_tuple(make_force(rng, 37, lo=9, hi=41))
     f = Pack(X, ELE, ind, dxdr=dX)
     NF, N = 37, 3 * 37
     Kref, dKref = k_total_device(_lib.RBF, 1.1, 0.6, 2.0, (None, f), None, use_tol=False, grad=True, symmetric=False)
+    y = torch.as_tensor(rng.normal(size=N), device="cuda")
+    noise = 0.05
+    full = _lml_eval(Kref, dKref, [(0, N)], 0, y, noise, noise)
+    # (a) the entries left of the diagonal are never read: NaN there gives the same bits
+    poisoned = torch.where(torch.triu(torch.ones(N, N, dtype=torch.bool, device="cuda")), dKref, float("nan"))
+    assert np.array_equal(_lml_eval(Kref, poisoned, [(0, N)], 0, y, noise, noise), full)
+    # (c) against the host
+    margin = _trace_vs_oracle(Kref, dKref, 0, y, noise, noise, full)
+    with capsys.disabled():
+        print("\n[lml_eval traces, force rows] max |err| / tol vs host = %.2e" % margin)
     for parts in (1, 2, 3):
         windows = gd.row_windows([], ind, parts, upper=True)
         assert windows[0][1][0] == 0 and windows[-1][1][1] == NF
@@ -213,24 +253,16 @@ def test_upper_mode_windows_symmetrize_and_trace():
         assert (K - Kref)[up].abs().max().item() <= 1e-13 * Kref.abs().max().item()
         _lib.call("gprb_symmetrize", ptr(K), N, N, stream())
         assert (K - Kref).abs().max().item() <= 1e-13 * Kref.abs().max().item()
-        # trace of (alpha alpha^T - Kinv) dK over all rows: full rows vs upper-only rows
-        alpha = torch.randn(N, dtype=torch.float64, device="cuda")
-        Kinv = torch.randn(N, N, dtype=torch.float64, device="cuda")
-        Kinv = Kinv + Kinv.T
-        out_full, out_up = (ctypes.c_double * 2)(), (ctypes.c_double * 2)()
-        _lib.call("gprb_lml_grad_trace", N, 0, N, ptr(alpha), ptr(Kinv), N, ptr(dKref), N, 0, 0.3, 0.7, 0, out_full, stream())
-        _lib.call("gprb_lml_grad_trace", N, 0, N, ptr(alpha), ptr(Kinv), N, ptr(dK), N, 0, 0.3, 0.7, 1, out_up, stream())
-        want = 0.5 * ((torch.outer(alpha, alpha) - Kinv) * dKref).sum().item()
-        assert abs(out_full[0] - want) <= 1e-10 * abs(want) and abs(out_up[0] - want) <= 1e-10 * abs(want)
-        assert abs(out_full[1] - out_up[1]) <= 1e-12 * abs(out_full[1])
+        # the FF_UPPER rows of dK (NaN left of the diagonal blocks) give the traces of the full dK
+        got = _lml_eval(Kref, dK, [(0, N)], 0, y, noise, noise)
+        assert np.all(np.abs(got[2:5] - full[2:5]) <= 1e-12 * np.abs(full[2:5]))
 
 
-def test_trace_sharded_mode_and_transpose():
-    """gprb_lml_grad_trace(upper_only=2) reads K_ee (upper), K_fe and K_ff (upper) only and must equal the full
-    trace; gprb_transpose_copy fills K_ef from K_fe."""
-    import ctypes
+def test_trace_sharded_mode_and_transpose(capsys):
+    """gprb_lml_eval reads K_ee (upper), K_fe and K_ff (upper) of dK only, and row ranges held by one rank give the traces of
+    the whole matrix; gprb_transpose_copy fills K_ef from K_fe."""
     from gpr_calculator_b200 import _lib
-    from gpr_calculator_b200.device import Pack, k_total_device, ptr, stream, c_vp
+    from gpr_calculator_b200.device import Pack, k_total_device, stream, c_vp
     from gpr_calculator_b200.utilities import list_to_tuple
     rng = np.random.default_rng(21)
     X, dX, ELE, ind = list_to_tuple(make_force(rng, 17, lo=5, hi=30))
@@ -238,26 +270,25 @@ def test_trace_sharded_mode_and_transpose():
     f, e = Pack(X, ELE, ind, dxdr=dX), Pack(Xe, Ee, inde)
     K, dK = k_total_device(_lib.RBF, 1.2, 0.7, 2.0, (e, f), None, use_tol=False, grad=True)
     NE, N = 6, 6 + 51
-    alpha = torch.randn(N, dtype=torch.float64, device="cuda")
-    W = torch.randn(N, N, dtype=torch.float64, device="cuda")
-    W = W + W.T
-    want = 0.5 * ((torch.outer(alpha, alpha) - W) * dK).sum().item()
+    y = torch.as_tensor(rng.normal(size=N), device="cuda")
+    noise_e, noise_f = 0.05, 0.1
+    full = _lml_eval(K, dK, [(0, N)], NE, y, noise_e, noise_f)
+    # (a) NaN in K_ef and left of the diagonal of K_ee and K_ff: never read, the same bits
     poisoned = dK.clone()
-    poisoned[:NE, NE:] = float("nan")                                    # K_ef: never read in mode 2
+    poisoned[:NE, NE:] = float("nan")
     poisoned[NE:, NE:] = torch.where(torch.triu(torch.ones(N - NE, N - NE, dtype=torch.bool, device="cuda")), dK[NE:, NE:],
                                      torch.full_like(dK[NE:, NE:], float("nan")))
     poisoned[:NE, :NE] = torch.where(torch.triu(torch.ones(NE, NE, dtype=torch.bool, device="cuda")), dK[:NE, :NE],
                                      torch.full_like(dK[:NE, :NE], float("nan")))
-    out = (ctypes.c_double * 2)()
-    _lib.call("gprb_lml_grad_trace", N, 0, N, ptr(alpha), ptr(W), N, ptr(poisoned), N, NE, 0.1, 0.2, 2, out, stream())
-    assert abs(out[0] - want) <= 1e-10 * abs(want)
-    # two row ranges, as a rank holds them
-    tot = 0.0
-    for r0, r1 in ((0, 2), (2, NE), (NE, NE + 21), (NE + 21, N)):
-        _lib.call("gprb_lml_grad_trace", N, r0, r1, ptr(alpha), ptr(W), N, c_vp(poisoned.data_ptr() + r0 * N * 8), N, NE,
-                  0.1, 0.2, 2, out, stream())
-        tot += out[0]
-    assert abs(tot - want) <= 1e-10 * abs(want)
+    assert np.array_equal(_lml_eval(K, poisoned, [(0, N)], NE, y, noise_e, noise_f), full)
+    # (b) four row ranges in one call, as a rank holds them (their rows stacked in dK_rows)
+    ranges = [(0, 2), (2, NE), (NE, NE + 21), (NE + 21, N)]
+    got = _lml_eval(K, poisoned, ranges, NE, y, noise_e, noise_f)
+    assert np.all(np.abs(got[2:5] - full[2:5]) <= 1e-12 * np.abs(full[2:5]))
+    # (c) against the host
+    margin = _trace_vs_oracle(K, dK, NE, y, noise_e, noise_f, full)
+    with capsys.disabled():
+        print("\n[lml_eval traces, energy + force rows] max |err| / tol vs host = %.2e" % margin)
     Kt = K.clone()
     Kt[:NE, NE:] = float("nan")
     _lib.call("gprb_transpose_copy", c_vp(Kt.data_ptr() + NE * 8), N, c_vp(Kt.data_ptr() + NE * N * 8), N, N - NE, NE, stream())

@@ -162,6 +162,11 @@ extern "C" int gprb_pack_create(gprb_pack **out, int n_groups, const int *group_
     GPRB_REQUIRE(ncols == 0 || ncols == 3, "gprb_pack_create: ncols must be 0 (energy) or 3 (force), got %d", ncols);
     GPRB_REQUIRE(norm_eps >= 0.0, "gprb_pack_create: norm_eps must be >= 0");
     GPRB_REQUIRE(ncols == 0 || dxdr_any != nullptr || n_groups == 0, "gprb_pack_create: dxdr is NULL for a force pack");
+    // the covariance kernels hold at most 2 * GPRB_MAX_KS k-steps of 4 (cov_mma.cu): refuse a pack none of them can use
+    if (d > 8 * GPRB_MAX_KS) {
+        gprb_set_error("gprb_pack_create: descriptor length %d > %d is not supported by the DMMA kernels", d, 8 * GPRB_MAX_KS);
+        return GPRB_ERR_UNSUPPORTED;
+    }
     { int rc0 = gprb_pool_init(); if (rc0) return rc0; }
     gprb_pack *p = new gprb_pack();
     p->stream = st;

@@ -55,6 +55,8 @@ long long gprb_launch_count(void);
  * with x^ = x/|x| and A~ = (I - x^ x^T) dxdr / |x|.  Rows with |x| <= 1e-8 are dropped as in
  * rbf_kernel.cpp:26,37.  group_rows_host[g] = number of rows of group g (the `indices` list).
  * x_any/dxdr_any/ele_any may be host or device pointers.
+ * The descriptor length d must be at most 64 (the longest the covariance kernels take); a longer one
+ * returns GPRB_ERR_UNSUPPORTED before any CUDA call, with *out = NULL.
  * norm_eps = 0 is the covariance convention.  norm_eps > 0 replaces |x| by |x| + norm_eps everywhere
  * and drops nothing: the convention of the numpy K_ff that Dot_mb.diag alone uses (Dot_mb.py:204-221). */
 int gprb_pack_create(gprb_pack **out, int n_groups, const int *group_rows_host, int d, int ncols,

@@ -433,10 +433,10 @@ def test_two_stage_path_matches_block_path(monkeypatch):
             assert (out["1"] - out[""]).abs().max().item() <= 1e-12 * scale
 
 
-def test_kee_tensor_path_species_blocks(oracle_libs, monkeypatch):
+def test_kee_tensor_path_species_blocks(oracle_libs):
     """K_ee on the DMMA tile path in the shape of the Pd4/MgO training set: large energy groups whose rows are ordered by
     species (tiles without a same-species pair are skipped, also when a group ends inside a skipped tile), ragged group
-    sizes, the symmetric training block and a rectangular window; against the C oracle and against the scalar kernel."""
+    sizes, the symmetric training block and a rectangular window; against the C oracle."""
     from gpr_calculator_b200.kernels import rbf_kernel as rk, dot_kernel as dk
     rng = np.random.default_rng(77)
     base = np.abs(rng.normal(size=30)) + 0.5
@@ -454,13 +454,9 @@ def test_kee_tensor_path_species_blocks(oracle_libs, monkeypatch):
     for a, b in ((E1, E1), (E1, E2), (E2, E1)):
         for zeta in (2.0, 3.0):
             ref = O.kee_C(a, b, 1.4, 0.35, zeta, grad=True)
-            monkeypatch.delenv("GPRB_KEE_SCALAR", raising=False)
             got = rk.kee_C(a, b, 1.4, 0.35, zeta, grad=True)
-            monkeypatch.setenv("GPRB_KEE_SCALAR", "1")
-            old = rk.kee_C(a, b, 1.4, 0.35, zeta, grad=True)
-            monkeypatch.delenv("GPRB_KEE_SCALAR", raising=False)
-            for x, y, z in zip(got, ref, old):
-                assert x.shape == y.shape and rel_err(x, y) <= TOL and rel_err(x, z) <= TOL, zeta
+            for x, y in zip(got, ref):
+                assert x.shape == y.shape and rel_err(x, y) <= TOL, zeta
             assert rel_err(dk.kee_C(a, b, 2.0, 1.5, zeta), OD.kee_C(a, b, 2.0, 1.5, zeta)) <= TOL
     K = rk.kee_C(E1, E1, 1.4, 0.35, 2.0)
     assert np.array_equal(K, K.T)

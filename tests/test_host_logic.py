@@ -377,3 +377,20 @@ def test_lml_eval_workspace_size():
     assert lib.gprb_lml_eval_work(32980, 340, 1, 16) == (340 + 2062) * 32980
     assert lib.gprb_lml_eval_work(172, 4, 1, 16) == (4 + 172) * 172          # one block: the whole matrix
     assert lib.gprb_lml_eval_work(32980, 340, 0, 16) == 0                    # no gradient: nothing to hold
+
+
+def test_pack_create_rejects_descriptors_longer_than_64():
+    """gprb_pack_create refuses d > 64 (no covariance kernel takes it) with GPRB_ERR_UNSUPPORTED before any CUDA call,
+    for energy and force packs whose other arguments are all valid."""
+    import ctypes
+    from gpr_calculator_b200 import _lib
+    lib = _lib.load()
+    rows = np.array([2, 3], dtype=np.int32)
+    ele = np.array([1, 1, 8, 8, 8], dtype=np.int32)
+    for d in (65, 72):
+        x = np.ones((5, d))
+        for ncols, dxdr in ((0, None), (3, np.ones((5, d, 3)))):
+            out = ctypes.c_void_p(0)
+            rc = lib.gprb_pack_create(ctypes.byref(out), 2, rows.ctypes.data, d, ncols, x.ctypes.data,
+                                      None if dxdr is None else dxdr.ctypes.data, ele.ctypes.data, 0.0, None)
+            assert rc == _lib.ERR_UNSUPPORTED and not out.value, (d, ncols, rc)

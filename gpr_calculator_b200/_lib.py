@@ -27,6 +27,8 @@ SIGNATURES = {
     "gprb_pack_destroy": (None, [c_vp]),
     "gprb_pack_info": (c_int, [c_vp, c_int_p, c_int_p, c_int_p, c_int_p, c_int_p]),
     "gprb_pack_pair_count": (c_ll, [c_vp, c_int, c_int, c_vp]),
+    "gprb_atom_plan_host": (c_int, [c_int, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "gprb_atom_plan_cost": (c_int, [c_int, c_vp, c_vp, c_int, c_int, c_vp, c_vp]),
     "gprb_kff": (c_int, [c_int, c_vp, c_vp, c_dbl, c_dbl, c_dbl, c_int, c_dbl, c_int, c_int, c_int,
                          c_vp, c_ll, c_vp, c_ll, c_vp]),
     "gprb_kef": (c_int, [c_int, c_vp, c_vp, c_dbl, c_dbl, c_dbl, c_int, c_int,

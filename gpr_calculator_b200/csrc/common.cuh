@@ -5,6 +5,7 @@
 #include <cstdarg>
 #include <vector>
 #include <map>
+#include <cstdint>
 #include "../../include/gpr_b200.h"
 
 #define GPRB_TILE_ROWS 8           // rows of one DMMA operand tile (M or N of mma.m8n8k4)
@@ -60,6 +61,13 @@ extern std::atomic<long long> g_gprb_launches;
 #define GPRB_CHUNK_TILES 4         // tiles per column chunk (one TMA stage)
 #define GPRB_REC_INTS 28           // 112 bytes: a multiple of 16 for cp.async.bulk
 
+struct gprb_atom_plan;               // atom plan of a force pack (cov_factored.cu)
+void gprb_atom_plan_free(gprb_atom_plan *plan, cudaStream_t st);
+// K_ff + dK/dl (RBF) of a force pack against itself, full window, one pre-zeroed destination, over the atoms its rows share
+// (cov_factored.cu); *done = false when the pairwise kernel is to run instead
+int gprb_kff_factored(gprb_pack *f, double p0, double p1, double zeta, int mode, double *K, long long ldk, double *dK,
+                      long long lddk, cudaStream_t st, bool *done);
+
 struct gprb_pack {
     int n_groups = 0, n_rows = 0, d = 0, ncols = 0, ncomp = 0, ks = 0, n_tiles = 0;
     int device = 0;
@@ -77,6 +85,10 @@ struct gprb_pack {
     int *tile_rec = nullptr;       // [n_tiles][GPRB_REC_INTS]
     int *d_row_ptr = nullptr;      // [G+1]
     int *d_group_rows = nullptr;   // [G]
+    uint64_t *row_hash = nullptr;  // [n_tiles*8]  hash of the raw x bits and the species code of each row (0 for padding)
+    // atom plan of the factored K_ff path (cov_factored.cu): built on the first call that can use it
+    gprb_atom_plan *plan = nullptr;
+    bool plan_tried = false;
     // cached row-side schedule for the last window used (see cov_mma.cu)
     int sched_g0 = -1, sched_g1 = -1, sched_n = 0;
     int4 *sched = nullptr;         // device [sched_n] {tile0, ntiles, entry_begin, n_entries}

@@ -35,13 +35,20 @@ extern "C" int gprb_device_info(int *sm_count, int *cc_major, int *cc_minor) {
     return GPRB_OK;
 }
 
+// splitmix64 finaliser
+__device__ __forceinline__ uint64_t mix64(uint64_t z) {
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    return z ^ (z >> 31);
+}
+
 // One warp per row of the flat tile layout (rows >= n_rows are tail padding).
 // HBM-bound: reads 8*d*(1+ncols) bytes and writes 8*4ks*(1+ncols) per row.
 __global__ void prep_rows_kernel(int n_padded, int n_rows, int d, int ncols, int ks, double norm_eps,
                                  const double *__restrict__ x, const double *__restrict__ dxdr,
                                  const int *__restrict__ ele,
                                  double *__restrict__ P, double *__restrict__ norm_out,
-                                 int *__restrict__ elep, int *__restrict__ tile_rec) {
+                                 int *__restrict__ elep, int *__restrict__ tile_rec, uint64_t *__restrict__ row_hash) {
     int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     int lane = threadIdx.x & 31;
     if (warp >= n_padded) return;
@@ -53,14 +60,21 @@ __global__ void prep_rows_kernel(int n_padded, int n_rows, int d, int ncols, int
     if (src < 0) {   // padding row
         for (int c = 0; c < ncomp; c++)
             for (int k = lane; k < kp; k += 32) Pt[((size_t)c * ks + (k >> 2)) * 32 + r * 4 + (k & 3)] = 0.0;
-        if (lane == 0) { norm_out[warp] = 0.0; elep[warp] = -1; tile_rec[(size_t)tile * GPRB_REC_INTS + r] = -1; }
+        if (lane == 0) { norm_out[warp] = 0.0; elep[warp] = -1; tile_rec[(size_t)tile * GPRB_REC_INTS + r] = -1; row_hash[warp] = 0; }
         return;
     }
     const double *xr = x + (size_t)src * d;
     double ss = 0.0;
-    for (int k = lane; k < d; k += 32) { double v = xr[k]; ss += v * v; }
+    uint64_t h = 0;                 // sum over k of mix(bits(x_k), k): equal rows hash equally (the atom plan's merge key)
+    for (int k = lane; k < d; k += 32) {
+        double v = xr[k];
+        ss += v * v;
+        h += mix64((uint64_t)__double_as_longlong(v) + (uint64_t)k * 0x9e3779b97f4a7c15ull);
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) h += __shfl_xor_sync(0xffffffffu, (unsigned long long)h, o);
     const double n = sqrt(ss) + norm_eps;
     const bool dropped = (norm_eps == 0.0) && !(n > GPRB_EPS_NORM);
     const double inv = dropped ? 0.0 : 1.0 / n;
@@ -90,6 +104,7 @@ __global__ void prep_rows_kernel(int n_padded, int n_rows, int d, int ncols, int
         const int code = dropped ? -(z + 2) : z;
         elep[warp] = code;
         tile_rec[(size_t)tile * GPRB_REC_INTS + r] = code;
+        row_hash[warp] = mix64(h ^ ((uint64_t)(uint32_t)code * 0xc2b2ae3d27d4eb4full));
     }
 }
 
@@ -148,7 +163,8 @@ extern "C" void gprb_pack_destroy(gprb_pack *p) {
     cudaStream_t st = p->stream;
     gprb_pool_free(p->P, st); gprb_pool_free(p->norm, st); gprb_pool_free(p->elep, st); gprb_pool_free(p->row_group, st);
     gprb_pool_free(p->tile_rec, st); gprb_pool_free(p->d_row_ptr, st); gprb_pool_free(p->d_group_rows, st);
-    gprb_pool_free(p->sched, st); gprb_pool_free(p->sched_ent, st);
+    gprb_pool_free(p->sched, st); gprb_pool_free(p->sched_ent, st); gprb_pool_free(p->row_hash, st);
+    gprb_atom_plan_free(p->plan, st);
     delete p;
 }
 
@@ -213,6 +229,7 @@ extern "C" int gprb_pack_create(gprb_pack **out, int n_groups, const int *group_
     PK_CUDA(cudaMallocAsync((void **)&p->norm, (size_t)n_padded * sizeof(double), st));
     PK_CUDA(cudaMallocAsync((void **)&p->elep, (size_t)n_padded * sizeof(int), st));
     PK_CUDA(cudaMallocAsync((void **)&p->row_group, (size_t)n_padded * sizeof(int), st));
+    PK_CUDA(cudaMallocAsync((void **)&p->row_hash, (size_t)n_padded * sizeof(uint64_t), st));
     PK_CUDA(cudaMallocAsync((void **)&p->tile_rec, rec.size() * sizeof(int), st));
     PK_CUDA(cudaMallocAsync((void **)&p->d_row_ptr, (size_t)(n_groups + 1) * sizeof(int), st));
     PK_CUDA(cudaMallocAsync((void **)&p->d_group_rows, (size_t)(n_groups > 0 ? n_groups : 1) * sizeof(int), st));
@@ -232,7 +249,7 @@ extern "C" int gprb_pack_create(gprb_pack **out, int n_groups, const int *group_
         const int threads = 256, wpb = threads / 32;
         const int blocks = (n_padded + wpb - 1) / wpb;
         prep_rows_kernel<<<blocks, threads, 0, st>>>(n_padded, p->n_rows, d, ncols, p->ks, norm_eps, dx, ddx, de,
-                                                     p->P, p->norm, p->elep, p->tile_rec);
+                                                     p->P, p->norm, p->elep, p->tile_rec, p->row_hash);
         GPRB_LAUNCHED();
         PK_CUDA(cudaGetLastError());
     }

@@ -63,6 +63,7 @@ SIGNATURES = {
     "gprb_so3_radial": (c_int, [c_int, c_vp, c_int, c_int, c_int, c_dbl, c_dbl, c_vp, c_vp, c_vp, c_vp]),
     "gprb_so3_power": (c_int, [c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_dbl, c_dbl, c_vp,
                                c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "gprb_virial_rows": (c_int, [c_int, c_int, c_vp, c_vp, c_vp, c_vp]),
 }
 
 

@@ -49,3 +49,25 @@ def rows_from_batch(r, centres=None, stress=False):
         dX = torch.cat((dX, voigt), dim=2)
     F = (x[cen], dX, numbers[cen].to(torch.int32), [int(v) for v in n_rows.cpu()])
     return E, F
+
+
+def virial_rows_from_batch(r):
+    """Rows of the total stress of every structure of the batch (descriptor created with stress=True).
+
+    The stress rows of rows_from_batch(stress=True) summed over all force items of a structure equal, centre by centre,
+    one row per atom with dxdr = sum over that atom's `seq` rows of rdxdr (gprb_virial_rows): the covariance is linear
+    in dxdr once x is fixed (DESIGN.md §2).  Returns (energy tuple as rows_from_batch, stress tuple (X [A,d], V [A,d,6],
+    ELE [A], indices = atoms per structure)) with V's columns in the order xx, yy, zz, xy, xz, yz."""
+    from . import _lib
+    from .device import ptr, stream
+    if r.get('rdxdr') is None:
+        raise ValueError("stress rows need a descriptor created with stress=True (rdxdr)")
+    x = r['x']
+    atom_ptr = r['atom_ptr'].long()
+    E = (x, r['numbers'].to(torch.int32), [int(v) for v in (atom_ptr[1:] - atom_ptr[:-1]).cpu()])
+    A, d = x.shape
+    seq_ptr = r['seq_ptr'].to(torch.int32).contiguous()
+    rdxdr = r['rdxdr'].contiguous()
+    V = torch.empty((A, d, 6), dtype=torch.float64, device=x.device)
+    _lib.call("gprb_virial_rows", A, d, ptr(seq_ptr), ptr(rdxdr), ptr(V), stream())
+    return E, (x, V, E[1], E[2])

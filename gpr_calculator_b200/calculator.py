@@ -6,6 +6,8 @@ structure and refits on the reference's cadence.  The keyword arguments (``base,
 stress, f_tol, return_std``), the result keys, the printed "From Base model" / "From Surrogate" lines
 and the abort on a bad refit are those of the reference.  With torch.distributed initialised, rank 0
 runs the base calculator and broadcasts the labels (replaces the mpi4py bcast of calculator.py:58-59,90-91).
+One keyword is added: ``stress_std=True`` (with ``stress=True``) also reports the standard deviation of the total
+stress as ``results['var_s']`` (``get_var_s()``); the gate does not read it.
 
 ASE is optional: with ASE installed ``GPR`` derives from ``ase.calculators.calculator.Calculator``;
 without it a minimal stand-in base class provides the same ``parameters`` / ``results`` protocol so
@@ -75,7 +77,7 @@ def _bcast(obj):
 
 
 class GPR(Calculator):
-    implemented_properties = ['energy', 'forces', 'stress', 'var_e', 'var_f']
+    implemented_properties = ['energy', 'forces', 'stress', 'var_e', 'var_f', 'var_s']
     nolabel = True
 
     def __init__(self, **kwargs):
@@ -158,14 +160,23 @@ class GPR(Calculator):
         stress = self.parameters.stress if 'stress' in self.parameters else False
         f_tol = self.parameters.f_tol if 'f_tol' in self.parameters else 1e-12
         return_std = self.parameters.return_std if 'return_std' in self.parameters else True
-        res = self.parameters.ff.predict_structure(atoms, stress, return_std, f_tol=f_tol)
-        if return_std:
+        stress_std = self.parameters.stress_std if 'stress_std' in self.parameters else False
+        if stress and stress_std:
+            # total stress and its standard deviation from one row per atom (GP.predict_structures(stress=True))
+            res = self.parameters.ff.predict_structures([atoms], return_std=True, f_tol=f_tol, stress=True)[0]
             self.results['var_e'] = res[3]
             self.results['var_f'] = res[4]
+            self.results['var_s'] = res[5]
+            self.results['stress'] = res[2]
+        else:
+            res = self.parameters.ff.predict_structure(atoms, stress, return_std, f_tol=f_tol)
+            if return_std:
+                self.results['var_e'] = res[3]
+                self.results['var_f'] = res[4]
+            self.results['stress'] = res[2].sum(axis=0) if stress else None
         self.results['energy'] = res[0]
         self.results['free_energy'] = res[0]
         self.results['forces'] = res[1]
-        self.results['stress'] = res[2].sum(axis=0) if stress else None
         self.forces = res[1]
 
     def get_var_e(self, total=False):
@@ -175,6 +186,10 @@ class GPR(Calculator):
 
     def get_var_f(self):
         return self.results["var_f"]
+
+    def get_var_s(self):
+        """Standard deviation [6] of the total stress (xx, yy, zz, xy, xz, yz); set when GPR(stress=True, stress_std=True)."""
+        return self.results["var_s"]
 
     def get_e(self, peratom=True):
         if peratom:

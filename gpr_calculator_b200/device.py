@@ -224,6 +224,35 @@ def k_total_stress_device(kernel, p0, p1, zeta, data1, data2, use_tol=True, tol=
     return K, interleave_stress(parts[0], parts[1], NF1)
 
 
+def virial_packs(data, norm_eps=0.0):
+    """Stress tuple of batch.virial_rows_from_batch (X, V [A, d, 6], ELE, indices) -> (force Pack of Voigt columns 0:3,
+    force Pack of columns 3:6): the total-stress counterpart of the two stress triples of stress_packs."""
+    X, V, ELE, indices = data
+    return tuple(Pack(X, ELE, indices, dxdr=V[:, :, a:a + 3], norm_eps=norm_eps) for a in (0, 3))
+
+
+def k_virial_device(kernel, p0, p1, zeta, packs, train_side, use_tol=True, tol=1e-10, zeta_ef=None, zeta_ff=None,
+                    prior_packs=None, prior_tol=1e-12):
+    """(K* [6 S, N2] with rows (structure, voigt 0..5), prior variance [6 S]) of the total stress of S structures.
+
+    packs: virial_packs of the structures; train_side: (energy Pack, force Pack).  K* takes the K_fe / K_ff arguments of
+    k_total_stress_device, so every row is the sum over atoms of that route's per-atom stress rows.  The prior is the
+    FF_DIAG of each triple with diag_device's conventions: prior_packs (default `packs`; the Dot kernel passes packs with
+    its norm_eps), `zeta` and prior_tol."""
+    require_cuda()
+    S = packs[0].n_groups
+    NE2, NF2 = _sizes(train_side)
+    n_cols = NE2 + 3 * NF2
+    parts, prior = [], []
+    for p, q in zip(packs, prior_packs or packs):
+        Ks = torch.empty((3 * S, n_cols), dtype=F64, device="cuda")
+        build_force_rows(kernel, p0, p1, zeta, (None, p), train_side, (0, S), Ks, None, use_tol=use_tol, tol=tol,
+                         zeta_ef=zeta_ef, zeta_ff=zeta_ff, ff_mode=_lib.FF_FULL)
+        parts.append(Ks)
+        prior.append(diag_device(kernel, p0, p1, zeta, (None, q), tol=prior_tol).reshape(-1, 1))
+    return interleave_stress(parts[0], parts[1], S), interleave_stress(prior[0], prior[1], S).reshape(-1)
+
+
 def packs_of(data):
     """dict {'energy':…, 'force':…} -> (energy Pack or None, force Pack or None)."""
     e = energy_pack(data["energy"]) if "energy" in data else None

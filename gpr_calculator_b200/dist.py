@@ -230,32 +230,42 @@ def all_reduce_array(values, device="cpu", group=None):
     return t.cpu().numpy()
 
 
-def gather_predictions(mine, n_atoms, first, return_std, device="cpu", group=None):
+def gather_predictions(mine, n_atoms, first, return_std, device="cpu", group=None, stress=False):
     """Combine per-rank prediction results into the full list on every rank.
 
     mine: this rank's results for the structures [first, first + len(mine)) of a list whose structures have
     n_atoms[k] atoms: tuples (E, F [n, 3], None) or (E, F, None, E_std, F_std [n, 3]).  Flat layout per structure:
-    E, F (3 n) [, E_std, F_std (3 n)]; every rank fills its own slots of a zero buffer, one all-reduce."""
+    E, F (3 n) [, E_std, F_std (3 n)]; every rank fills its own slots of a zero buffer, one all-reduce.
+    stress=True: tuples (E, F, S [6]) or (E, F, S, E_std, F_std, S_std [6]); S follows F and S_std follows F_std."""
     width = 2 if return_std else 1
-    sizes = np.array([(1 + 3 * n) * width for n in n_atoms], dtype=np.int64)
+    ns = 6 if stress else 0
+    sizes = np.array([(1 + 3 * n + ns) * width for n in n_atoms], dtype=np.int64)
     offs = np.concatenate(([0], np.cumsum(sizes)))
     flat = np.zeros(int(offs[-1]))
     for k, res in enumerate(mine):
         o, n3 = int(offs[first + k]), 3 * n_atoms[first + k]
+        h = 1 + n3 + ns                      # start of the standard deviations
         flat[o] = res[0]
         flat[o + 1:o + 1 + n3] = np.asarray(res[1]).reshape(-1)
+        if stress:
+            flat[o + 1 + n3:o + h] = res[2]
         if return_std:
-            flat[o + 1 + n3] = res[3]
-            flat[o + 2 + n3:o + 2 + 2 * n3] = np.asarray(res[4]).reshape(-1)
+            flat[o + h] = res[3]
+            flat[o + h + 1:o + h + 1 + n3] = np.asarray(res[4]).reshape(-1)
+            if stress:
+                flat[o + h + 1 + n3:o + 2 * h] = res[5]
     flat = all_reduce_array(flat, device=device, group=group)
     out = []
     for k, n in enumerate(n_atoms):
         o, n3 = int(offs[k]), 3 * n
+        h = 1 + n3 + ns
         F = flat[o + 1:o + 1 + n3].reshape(-1, 3).copy()
+        S = flat[o + 1 + n3:o + h].copy() if stress else None
         if return_std:
-            out.append((float(flat[o]), F, None, float(flat[o + 1 + n3]), flat[o + 2 + n3:o + 2 + 2 * n3].reshape(-1, 3).copy()))
+            res = (float(flat[o]), F, S, float(flat[o + h]), flat[o + h + 1:o + h + 1 + n3].reshape(-1, 3).copy())
+            out.append(res + ((flat[o + h + 1 + n3:o + 2 * h].copy(),) if stress else ()))
         else:
-            out.append((float(flat[o]), F, None))
+            out.append((float(flat[o]), F, S))
     return out
 
 

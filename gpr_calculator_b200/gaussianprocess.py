@@ -961,14 +961,17 @@ class GP():
             return E, F, S, E_std, F_std
         return E, F, S
 
+    def _require_stress_descriptor(self):
+        if not getattr(self.descriptor, "stress", False) or not hasattr(self.descriptor, "calculate_batch"):
+            raise ValueError("predict_structure(stress=True) needs a descriptor created with stress=True "
+                             "(the reference reads d['rdxdr'], gaussianprocess.py:862)")
+
     def _predict_structure_stress(self, struc, return_std, f_tol):
         """predict_structure(stress=True): K* rows of the energy, of all 3 n force components and of the
         6 n Voigt stress components (k_total_with_stress), mean = K* alpha."""
         from .batch import rows_from_batch
         from .device import energy_pack, stress_packs
-        if not getattr(self.descriptor, "stress", False) or not hasattr(self.descriptor, "calculate_batch"):
-            raise ValueError("predict_structure(stress=True) needs a descriptor created with stress=True "
-                             "(the reference reads d['rdxdr'], gaussianprocess.py:862)")
+        self._require_stress_descriptor()
         n = len(struc)
         fixed = set(self._get_fixed_atoms(struc))
         free_ids = [i for i in range(n) if i not in fixed]
@@ -999,7 +1002,7 @@ class GP():
             return E, F, S, y_std[0], F_std
         return E, F, S
 
-    def predict_structures(self, strucs, return_std=False, f_tol=1e-8, batch=32, shard=True):
+    def predict_structures(self, strucs, return_std=False, f_tol=1e-8, batch=32, shard=True, stress=False):
         """Batched predict_structure(stress=False): descriptors, K*, mean and variance of `batch`
         structures per device pass (the "predict 10k structures" path of the benchmark).
 
@@ -1010,19 +1013,27 @@ class GP():
         gaussianprocess.py:834-918 under mpi4py).  shard=False: every rank predicts the whole list (replicas).
 
         Returns a list of (E, F, None) or (E, F, None, E_std, F_std) tuples, one per structure, equal to
-        what predict_structure returns for each of them."""
+        what predict_structure returns for each of them.
+
+        stress=True (descriptor created with stress=True) also predicts each structure's total stress S [6] (xx, yy, zz,
+        xy, xz, yz; predict_structure(stress=True)[2].sum(axis=0), what GPR reports as `stress`) and, with return_std, its
+        standard deviation S_std [6]: tuples (E, F, S) or (E, F, S, E_std, F_std, S_std).  The stress rows are one row
+        per atom (batch.virial_rows_from_batch) in a K* of their own, so E and F are those of stress=False."""
         require_cuda()
         if self.base_potential is not None:
             raise NotImplementedError("base potentials are outside the B200 hot path")
+        if stress:
+            self._require_stress_descriptor()
         rank, size = gdist.world()
         if size == 1 or not shard or len(strucs) == 0:
-            return self._predict_structures_local(strucs, return_std, f_tol, batch)
+            return self._predict_structures_local(strucs, return_std, f_tol, batch, stress)
         bounds = gdist.split_groups([len(s_) for s_ in strucs], size)
-        mine = self._predict_structures_local(strucs[bounds[rank]:bounds[rank + 1]], return_std, f_tol, batch)
-        return gdist.gather_predictions(mine, [len(s_) for s_ in strucs], bounds[rank], return_std, device="cuda")
+        mine = self._predict_structures_local(strucs[bounds[rank]:bounds[rank + 1]], return_std, f_tol, batch, stress)
+        return gdist.gather_predictions(mine, [len(s_) for s_ in strucs], bounds[rank], return_std, device="cuda",
+                                        stress=stress)
 
-    def _predict_structures_local(self, strucs, return_std, f_tol, batch):
-        from .batch import rows_from_batch
+    def _predict_structures_local(self, strucs, return_std, f_tol, batch, stress=False):
+        from .batch import rows_from_batch, virial_rows_from_batch
         train_x = self.get_train_x()
         out = []
         for s0 in range(0, len(strucs), batch):
@@ -1031,24 +1042,31 @@ class GP():
             for st_ in part:
                 fixed = set(self._get_fixed_atoms(st_))
                 free.append([i for i in range(len(st_)) if i not in fixed])
-            E_t, F_t = rows_from_batch(self.descriptor.calculate_batch(part, to_host=False), free)
+            r = self.descriptor.calculate_batch(part, to_host=False)
+            E_t, F_t = rows_from_batch(r, free)
             data = {"energy": E_t}
             if F_t is not None:
                 data["force"] = F_t
             _, mean, var = self._predict_device(data, train_x, f_tol, return_std)
             y = mean.cpu().numpy()
             sd = np.sqrt(var.cpu().numpy()) if return_std else None
+            if stress:
+                K_s, prior_s = self.kernel.k_virial_device(virial_rows_from_batch(r)[1], train_x, tol=f_tol)
+                mean_s, var_s = self._mean_var(K_s, prior_s if return_std else None)
+                y_s = mean_s.cpu().numpy().reshape(len(part), 6)
+                sd_s = np.sqrt(var_s.cpu().numpy()).reshape(len(part), 6) if return_std else None
             pos = len(part)
             for k, st_ in enumerate(part):
                 n, nf = len(st_), len(free[k])
                 F = np.zeros((n, 3))
                 F[free[k]] = y[pos:pos + 3 * nf].reshape(nf, 3)
+                S = y_s[k] if stress else None
                 if return_std:
                     F_std = np.zeros((n, 3))
                     F_std[free[k]] = sd[pos:pos + 3 * nf].reshape(nf, 3)
-                    out.append((y[k] * n, F, None, sd[k], F_std))
+                    out.append((y[k] * n, F, S, sd[k], F_std) + ((sd_s[k],) if stress else ()))
                 else:
-                    out.append((y[k] * n, F, None))
+                    out.append((y[k] * n, F, S))
                 pos += 3 * nf
         return out
 

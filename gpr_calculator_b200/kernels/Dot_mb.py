@@ -14,7 +14,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..device import packs_of, k_total_device, k_total_stress_device, diag_device, energy_pack, force_pack
+from ..device import (packs_of, k_total_device, k_total_stress_device, diag_device, energy_pack, force_pack,
+                      k_virial_device, virial_packs)
 
 
 class Dot_mb():
@@ -92,6 +93,13 @@ class Dot_mb():
         # same zeta-in-the-sigma0-slot quirk as k_total: the cross blocks use zeta = 2 (Dot_mb.py:166-170)
         return k_total_stress_device(_lib.DOT, float(self.sigma), float(self.sigma0), float(self.zeta), data1, data2,
                                      use_tol=False, tol=0.0, zeta_ef=2.0, zeta_ff=2.0)
+
+    def k_virial_device(self, V, data2, tol=1e-10):
+        """(K*, prior variance) of the total stress rows of V: K* with k_total_stress_device's cross-block zeta = 2, the
+        prior as diag_device builds force rows (norm_eps = 1e-8, self.zeta)."""
+        return k_virial_device(_lib.DOT, float(self.sigma), float(self.sigma0), float(self.zeta), virial_packs(V),
+                               packs_of(data2), use_tol=False, tol=0.0, zeta_ef=2.0, zeta_ff=2.0,
+                               prior_packs=virial_packs(V, norm_eps=1e-8), prior_tol=0.0)
 
     def k_total_with_stress(self, data1, data2, tol=1e-10):
         """Dot_mb.py:150-173 (tol is not used there either)."""

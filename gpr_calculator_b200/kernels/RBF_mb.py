@@ -11,7 +11,7 @@ GP.predict use so that K never leaves HBM).  The reference's mpi4py row split
 import numpy as np
 
 from .. import _lib
-from ..device import packs_of, k_total_device, k_total_stress_device, diag_device
+from ..device import packs_of, k_total_device, k_total_stress_device, diag_device, k_virial_device, virial_packs
 
 
 class RBF_mb():
@@ -86,6 +86,12 @@ class RBF_mb():
         """(K, K1) as CUDA tensors; K1 holds the 6 Voigt stress rows of every force item of data1."""
         return k_total_stress_device(_lib.RBF, float(self.sigma), float(self.l), float(self.zeta), data1, data2,
                                      use_tol=True, tol=tol)
+
+    def k_virial_device(self, V, data2, tol=1e-10):
+        """(K*, prior variance) of the total stress rows of the stress tuple V (batch.virial_rows_from_batch): K* with the
+        pair cut of k_total_stress_device, the prior with the force-row tol of diag_device."""
+        return k_virial_device(_lib.RBF, float(self.sigma), float(self.l), float(self.zeta), virial_packs(V), packs_of(data2),
+                               use_tol=True, tol=tol, prior_tol=1e-12)
 
     def k_total_with_stress(self, data1, data2, tol=1e-10):
         """Covariance for energy / force / stress prediction (RBF_mb.py:206-229): data1's force items carry

@@ -265,6 +265,13 @@ int gprb_so3_power(int n_atoms, const int *nb_ptr, const int *nb_j, const double
                    double *x, double *dxdr, long long *seq,
                    const double *pos, const double *inv_vol, double *rdxdr, void *stream);
 
+/* gprb_virial_rows : strain derivative of every atom's descriptor, the row of that atom in its structure's
+ *   total-stress group:  out[a, k, v] = sum_{q in [seq_ptr[a], seq_ptr[a+1])} rdxdr[q, k, voigt(v)]
+ *   with v = xx, yy, zz, xy, xz, yz; seq_ptr[n_atoms + 1] and rdxdr[n_seq, d, 3, 3] as gprb_so3_power writes them,
+ *   out [n_atoms, d, 6].  Each entry is summed by one thread in increasing q (bitwise reproducible).
+ *   GPRB_ERR_ARG for n_atoms < 0, d outside [1, 64] or a NULL pointer (n_atoms > 0). */
+int gprb_virial_rows(int n_atoms, int d, const int *seq_ptr_dev, const double *rdxdr_dev, double *out_dev, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -67,6 +67,11 @@ void gprb_atom_plan_free(gprb_atom_plan *plan, cudaStream_t st);
 // (cov_factored.cu); *done = false when the pairwise kernel is to run instead
 int gprb_kff_factored(gprb_pack *f, double p0, double p1, double zeta, int mode, double *K, long long ldk, double *dK,
                       long long lddk, cudaStream_t st, bool *done);
+// K_fe / K_ef + dK/dl (RBF) of a force pack against an energy pack, full window, one destination, outputs zeroed by the
+// caller, over the atoms the force pack's rows share (cov_factored.cu); *done = false when the pairwise kernel is to run
+int gprb_kef_factored(const gprb_pack *e, gprb_pack *f, double p0, double p1, double zeta, double *Kef, long long ld_ef,
+                      double *Kfe, long long ld_fe, double *dKef, long long ld_def, double *dKfe, long long ld_dfe,
+                      cudaStream_t st, bool *done);
 
 struct gprb_pack {
     int n_groups = 0, n_rows = 0, d = 0, ncols = 0, ncomp = 0, ks = 0, n_tiles = 0;

@@ -18,6 +18,13 @@
 //   kff_contract_kernel [K | dK](3I+c, 3J+e) = Acal_S . [Z | Z']^T, stored with the UPPER / SYMMETRIC rules of cov_mma.cu
 // Both are FP64 m8n8k4 MMA kernels; every output entry is written by exactly one thread with a fixed summation order, so
 // the build is bitwise reproducible.
+//
+// K_fe / K_ef with dK/dl regroup the same way over the force side's atoms (the energy side needs no plan): for energy group
+// I (rows a) and force group J of cluster T,
+//     K_fe(3J+c, I) = -(1/n_I) sum_k A~_c(J,k) . Y_I(k)      Y_I(k) = sum_{a in I} W1(a,k) x^(a)
+// and dK/dl with Y' built from U1.  Per cluster T, in batches of clusters that bound the workspace:
+//   kef_y_kernel                 s, the weights, then Y and Y' -> workspace [2 NE] x [npad_T * 32]
+//   kff_contract_kernel<true>    [K_fe | dK_fe](3J+c, I) = Acal_T . [Y | Y']^T, stored to K_fe, K_ef and their dK/dl
 #include "cov_common.cuh"
 #include <cstdlib>
 #include <cstring>
@@ -55,6 +62,7 @@ struct gprb_atom_plan {
     double *Acal = nullptr;
     PairList lists[2];                    // [0] S <= T (UPPER, SYMMETRIC), [1] every pair (FULL)
     double pairwise_dmma[2] = {0, 0}, factored_dmma[2] = {0, 0};
+    std::vector<int> cgrp, cslots;        // host copies of gprb_atom_plan_host's cluster_grp / cluster_slots (K_ef cost)
 };
 
 void gprb_atom_plan_free(gprb_atom_plan *pl, cudaStream_t st) {
@@ -157,6 +165,21 @@ void plan_costs(int n_clusters, const int *cluster_grp, const int *cluster_slots
     *factored = f;
 }
 
+// The same for K_fe + dK/dl against an energy pack of ne_rows rows in ne groups.  Pairwise (cov_mma_kernel<1, 8, RBF,
+// grad>): 32 per pair of 8-row tiles (4 component tiles x 8 k-steps).  Factored, per cluster T: kef_y_kernel 24 per
+// (energy tile, 8 slots of T); kff_contract_kernel<true> (3 m_T / 8)(2 NE / 8)(8 npad_T).
+void plan_costs_kef(int n_clusters, const int *cluster_grp, const int *cluster_slots, int n_rows, int ne_rows, int ne,
+                    double *pairwise, double *factored) {
+    const double etiles = (double)((ne_rows + 7) / 8);
+    *pairwise = 32.0 * (double)((n_rows + 7) / 8) * etiles;
+    double f = 0.0;
+    for (int T = 0; T < n_clusters; T++) {
+        const double nt = pad8(cluster_slots[T]), mt = cluster_grp[T + 1] - cluster_grp[T];
+        f += 24.0 * etiles * (nt / 8) + std::ceil(3 * mt / 8) * std::ceil(2.0 * ne / 8) * 8 * nt;
+    }
+    *factored = f;
+}
+
 }  // namespace
 
 extern "C" int gprb_atom_plan_cost(int n_clusters, const int *cluster_grp, const int *cluster_slots, int n_rows, int upper,
@@ -164,6 +187,16 @@ extern "C" int gprb_atom_plan_cost(int n_clusters, const int *cluster_grp, const
     GPRB_REQUIRE(n_clusters >= 0 && (n_clusters == 0 || (cluster_grp && cluster_slots)) && pairwise_dmma && factored_dmma,
                  "gprb_atom_plan_cost: NULL argument");
     plan_costs(n_clusters, cluster_grp, cluster_slots, n_rows, upper, pairwise_dmma, factored_dmma);
+    return GPRB_OK;
+}
+
+extern "C" int gprb_atom_plan_cost_kef(int n_clusters, const int *cluster_grp, const int *cluster_slots, int n_rows,
+                                       int n_energy_rows, int n_energy_groups, double *pairwise_dmma, double *factored_dmma) {
+    GPRB_REQUIRE(n_clusters >= 0 && (n_clusters == 0 || (cluster_grp && cluster_slots)) && pairwise_dmma && factored_dmma,
+                 "gprb_atom_plan_cost_kef: NULL argument");
+    GPRB_REQUIRE(n_rows >= 0 && n_energy_rows >= 0 && n_energy_groups >= 0, "gprb_atom_plan_cost_kef: negative size");
+    plan_costs_kef(n_clusters, cluster_grp, cluster_slots, n_rows, n_energy_rows, n_energy_groups, pairwise_dmma,
+                   factored_dmma);
     return GPRB_OK;
 }
 
@@ -304,27 +337,116 @@ __global__ void __launch_bounds__(128) kff_z_kernel(const FactArgs A, const CovP
                     make_double2(Z[w][e][t][0], Z[w][e][t][1]);
 }
 
+// Energy side of the K_ef build: the energy pack's x^ slab (one component, ks = 8) in flat 8-row tiles and its groups.
+struct KefE { const double *P; const int *elep; const int *row_ptr; int ne; };
+
+// CTA = (energy group I, cluster T0 + blockIdx.y, up to 4 tiles of 8 slots of T); warp = one 8-slot tile k of T, all 32
+// columns d.  Per energy tile holding rows of I: s^T = X^_T . x^_a^T (8 DMMAs) with the slots as A operand, the weights of
+// this thread's two (k, a) pairs (rows of other groups masked), then Y += W1 x^ and Y' += U1 x^ (16): the accumulator
+// fragment of s^T is the A fragment of the second product with the row order a = 2 q4 + jj.  A tile shared by two groups
+// is multiplied once for each.
+template <int ZI>
+__global__ void __launch_bounds__(128) kef_y_kernel(const FactArgs A, const CovParams P, const KefE E, int T0) {
+    __shared__ double sTab[EXP_TAB];
+    if (threadIdx.x < EXP_TAB) sTab[threadIdx.x] = d_exp2_tab[threadIdx.x];
+    __syncthreads();
+    const int I = blockIdx.x, T = T0 + blockIdx.y;
+    const ClusterDev cT = A.cl[T];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, ra = lane >> 2, q4 = lane & 3;
+    const int kt = blockIdx.z * 4 + warp;
+    if (kt * 8 >= cT.npad) return;
+
+    double xa[8];
+    {
+        const double *XT = A.Xh + (size_t)(cT.slot0 + kt * 8 + ra) * 32 + q4;
+#pragma unroll
+        for (int ks = 0; ks < 8; ks++) xa[ks] = XT[4 * ks];
+    }
+    const int ek = A.spec[cT.slot0 + kt * 8 + ra];
+    const int r0 = E.row_ptr[I], r1 = E.row_ptr[I + 1];
+    double Y[2][4][2];
+#pragma unroll
+    for (int w = 0; w < 2; w++)
+#pragma unroll
+        for (int t = 0; t < 4; t++) { Y[w][t][0] = 0.0; Y[w][t][1] = 0.0; }
+
+    for (int tile = r0 >> 3; tile * 8 < r1; tile++) {
+        const double *pe = E.P + (size_t)tile * GPRB_MAX_KS * 32;     // fragment (k-step ks) = pe[32 ks + lane]
+        double s[2] = {0.0, 0.0};
+#pragma unroll
+        for (int ks = 0; ks < 8; ks++) dmma(s[0], s[1], xa[ks], pe[32 * ks + lane]);
+#pragma unroll
+        for (int jj = 0; jj < 2; jj++) {
+            const int a = tile * 8 + 2 * q4 + jj;
+            bool valid = a >= r0 && a < r1 && ek >= 0 && ek == E.elep[a];
+            double w1 = 0.0, w2 = 0.0, u1 = 0.0, u2 = 0.0;
+            pair_weights<GPRB_KERNEL_RBF, true, false, ZI>(P, sTab, s[jj], valid, w1, w2, u1, u2);
+            const double W1 = valid ? w1 : 0.0, U1 = valid ? u1 : 0.0;
+#pragma unroll
+            for (int t = 0; t < 4; t++) {
+                // B fragment element (k = q4, n = ra) is x^(a)[8 t + ra]: k-step 2 t + ra / 4, entry ra % 4 of row 2 q4 + jj
+                const double bx = pe[(2 * t + (ra >> 2)) * 32 + (2 * q4 + jj) * 4 + (ra & 3)];
+                dmma(Y[0][t][0], Y[0][t][1], W1, bx);
+                dmma(Y[1][t][0], Y[1][t][1], U1, bx);
+            }
+        }
+    }
+    // Y rows: [w][I] of the cluster's [2 NE] x [npad_T * 32] block (row-major, the contraction's B operand)
+    const size_t ldy = (size_t)cT.npad * 32;
+    double *yp = A.Zw + (size_t)2 * E.ne * 32 * (cT.slot0 - A.cl[T0].slot0) + (size_t)(kt * 8 + ra) * 32 + 2 * q4;
+#pragma unroll
+    for (int w = 0; w < 2; w++)
+#pragma unroll
+        for (int t = 0; t < 4; t++)
+            *reinterpret_cast<double2 *>(yp + (size_t)(w * E.ne + I) * ldy + 8 * t) = make_double2(Y[w][t][0], Y[w][t][1]);
+}
+
 constexpr int CT = 64, CK = 32, SST = CK + 4;      // CTA tile, k chunk, shared-memory row stride (conflict-free fragments)
 constexpr size_t CONTRACT_SMEM = (size_t)2 * 2 * CT * SST * sizeof(double);
+
+// Outputs of kff_contract_kernel.  K_ff: K / dK with the UPPER / SYMMETRIC / FULL rules of `mode`.  K_ef: K = K_fe,
+// dK = dK_fe/dl ([3 NF] x [NE]), K2 = K_ef, dK2 = dK_ef/dl ([NE] x [3 NF]), each written when not NULL.
+struct ContractOut {
+    double *K, *dK, *K2, *dK2;
+    long long ldk, lddk, ldk2, lddk2;
+    int mode, ne;
+    const int *group_rowsE;          // K_ef: rows per energy group (the pairwise epilogue's -1 / n_I)
+};
 
 __device__ __forceinline__ void cp_async16(void *dst, const void *src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src) : "memory");
 }
 
-// C [3 m_S] x [6 m_T] = Acal_S . Zw^T (K-dimension npad_S * 32); CTA tile 64 x 64, 4 warps of 32 x 32, 2-stage cp.async ring.
-// Column n < 3 m_T is K(3I+c, 3J+e), the rest dK/dl.  UPPER / SYMMETRIC: group blocks J >= I only (and their mirror).
-__global__ void __launch_bounds__(128) kff_contract_kernel(const FactArgs A, int p0, int mode, double *K, long long ldk,
-                                                           double *dK, long long lddk) {
+// C [3 m_S] x [N] = Acal_S . Zw^T (K-dimension npad_S * 32); CTA tile 64 x 64, 4 warps of 32 x 32, 2-stage cp.async ring.
+// Grid: (unit, m tile, n tile).  K_ff (KEF = false): unit = cluster pair p0 + u (S, T), N = 6 m_T; column n < 3 m_T is K(3I+c, 3J+e), the rest dK/dl;
+// UPPER / SYMMETRIC: group blocks J >= I only (and their mirror).
+// K_ef (KEF = true): unit = cluster S = p0 + u, N = 2 NE; column n < NE is K_fe(3J+c, n), the rest dK_fe/dl.
+template <bool KEF>
+__global__ void __launch_bounds__(128) kff_contract_kernel(const FactArgs A, int p0, const ContractOut O) {
     extern __shared__ __align__(16) double smem_c[];
-    const int2 st = A.pairs[p0 + blockIdx.x];
-    const ClusterDev cS = A.cl[st.x], cT = A.cl[st.y];
-    const int M = 3 * cS.m, N = 6 * cT.m, Kd = cS.npad * 32;
+    const int u = blockIdx.x;
+    int S, N;
+    const double *Bb;
+    ClusterDev cT = {};
+    if (KEF) {
+        S = p0 + u;
+        N = 2 * O.ne;
+        Bb = A.Zw + (size_t)2 * O.ne * 32 * (A.cl[S].slot0 - A.cl[p0].slot0);
+    } else {
+        const int2 st = A.pairs[p0 + u];
+        S = st.x;
+        cT = A.cl[st.y];
+        N = 6 * cT.m;
+        Bb = A.Zw + A.zoff[p0 + u];
+    }
+    const ClusterDev cS = A.cl[S];
+    const int M = 3 * cS.m, Kd = cS.npad * 32;
     const int m0 = blockIdx.y * CT, n0 = blockIdx.z * CT;
     if (m0 >= M || n0 >= N) return;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, ra = lane >> 2, q4 = lane & 3;
     const int wm = warp >> 1, wn = warp & 1;
     const bool active = m0 + 32 * wm < M && n0 + 32 * wn < N;
-    const double *Ab = A.Acal + cS.aoff, *Bb = A.Zw + A.zoff[p0 + blockIdx.x];
+    const double *Ab = A.Acal + cS.aoff;
     double *sA = smem_c, *sB = smem_c + 2 * CT * SST;
 
     auto load = [&](int buf, int k0) {
@@ -369,7 +491,7 @@ __global__ void __launch_bounds__(128) kff_contract_kernel(const FactArgs A, int
         __syncthreads();
     }
     if (!active) return;
-    const int mT3 = 3 * cT.m;
+    const int nG = KEF ? O.ne : 3 * cT.m;       // columns per output (K, then dK/dl)
 #pragma unroll
     for (int i = 0; i < 4; i++) {
         const int r = m0 + 32 * wm + 8 * i + ra;
@@ -381,14 +503,23 @@ __global__ void __launch_bounds__(128) kff_contract_kernel(const FactArgs A, int
             for (int h = 0; h < 2; h++) {
                 const int n = n0 + 32 * wn + 8 * j + 2 * q4 + h;
                 if (n >= N) continue;
-                const bool grad = n >= mT3;
-                const int nn = grad ? n - mT3 : n;
-                const int J = cT.grp0 + nn / 3, e = nn % 3;
-                double *dst = grad ? dK : K;
-                const long long ld = grad ? lddk : ldk;
+                const bool grad = n >= nG;
+                const int nn = grad ? n - nG : n;
                 const double v = acc[i][j][h];
-                if (mode == GPRB_FF_FULL || J >= I) dst[(long long)(3 * I + c) * ld + 3 * J + e] = v;
-                if (mode == GPRB_FF_SYMMETRIC && J > I) dst[(long long)(3 * J + e) * ld + 3 * I + c] = v;
+                if (KEF) {
+                    // force group I, energy group nn: K_fe = -(1 / n_nn) sum, as the pairwise NB = 1 epilogue
+                    const int nE = O.group_rowsE[nn];
+                    const double val = nE > 0 ? -v / (double)nE : 0.0;
+                    double *fe = grad ? O.dK : O.K, *ef = grad ? O.dK2 : O.K2;
+                    if (fe) fe[(long long)(3 * I + c) * (grad ? O.lddk : O.ldk) + nn] = val;
+                    if (ef) ef[(long long)nn * (grad ? O.lddk2 : O.ldk2) + 3 * I + c] = val;
+                } else {
+                    const int J = cT.grp0 + nn / 3, e = nn % 3;
+                    double *dst = grad ? O.dK : O.K;
+                    const long long ld = grad ? O.lddk : O.ldk;
+                    if (O.mode == GPRB_FF_FULL || J >= I) dst[(long long)(3 * I + c) * ld + 3 * J + e] = v;
+                    if (O.mode == GPRB_FF_SYMMETRIC && J > I) dst[(long long)(3 * J + e) * ld + 3 * I + c] = v;
+                }
             }
     }
 }
@@ -514,6 +645,8 @@ int build_plan(gprb_pack *f, cudaStream_t st, gprb_atom_plan **out) {
     gprb_pool_free(d_gd, st); gprb_pool_free(d_first, st); gprb_pool_free(d_next, st);
     for (int u = 0; u < 2; u++)
         plan_costs(nc, cgrp.data(), cslots.data(), R, u == 0, &pl->pairwise_dmma[u], &pl->factored_dmma[u]);
+    pl->cgrp.assign(cgrp.begin(), cgrp.begin() + nc + 1);
+    pl->cslots.assign(cslots.begin(), cslots.begin() + nc);
     // the host vectors die at return: make the pageable copies explicit and surface faults of the plan kernels here
     FP_CUDA(cudaStreamSynchronize(st));
     *out = pl;
@@ -554,22 +687,29 @@ int build_pairs(gprb_atom_plan *pl, int kind, cudaStream_t st) {
 
 constexpr int MAX_DEV_F = 64;
 
-template <int ZI>
-int run_batches(gprb_atom_plan *pl, PairList &L, const CovParams &P, int mode, double *K, long long ldk, double *dK,
-                long long lddk, cudaStream_t st) {
+template <bool KEF>
+int contract_config() {
     static bool configured[MAX_DEV_F] = {};
     int dev = 0;
     GPRB_CUDA(cudaGetDevice(&dev));
     if (dev >= 0 && dev < MAX_DEV_F && !configured[dev]) {
-        GPRB_CUDA(cudaFuncSetAttribute(kff_contract_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONTRACT_SMEM));
+        GPRB_CUDA(cudaFuncSetAttribute(kff_contract_kernel<KEF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)CONTRACT_SMEM));
         configured[dev] = true;
     }
+    return GPRB_OK;
+}
+
+template <int ZI>
+int run_batches(gprb_atom_plan *pl, PairList &L, const CovParams &P, const ContractOut &O, cudaStream_t st) {
+    int rc = contract_config<false>();
+    if (rc) return rc;
     FactArgs A = {pl->d_cl, L.d_pairs, L.d_zoff, pl->Xh, pl->spec, pl->Acal, nullptr};
     GPRB_CUDA(cudaMallocAsync((void **)&A.Zw, (size_t)L.max_zdoubles * sizeof(double), st));
     for (const Batch &b : L.batches) {
         kff_z_kernel<ZI><<<dim3(b.np, b.max_mt, b.max_jb), 128, 0, st>>>(A, P, b.p0);
         GPRB_LAUNCHED();
-        kff_contract_kernel<<<dim3(b.np, b.max_mb, b.max_nb), 128, CONTRACT_SMEM, st>>>(A, b.p0, mode, K, ldk, dK, lddk);
+        kff_contract_kernel<false><<<dim3(b.np, b.max_mb, b.max_nb), 128, CONTRACT_SMEM, st>>>(A, b.p0, O);
         GPRB_LAUNCHED();
     }
     const cudaError_t e = cudaGetLastError();
@@ -578,36 +718,119 @@ int run_batches(gprb_atom_plan *pl, PairList &L, const CovParams &P, int mode, d
     return GPRB_OK;
 }
 
+// K_ef: batches of consecutive clusters whose Y workspace stays within WS_BYTES (and 65535 clusters: grid y)
+template <int ZI>
+int run_kef(gprb_atom_plan *pl, const KefE &E, const CovParams &P, const ContractOut &O, cudaStream_t st) {
+    int rc = contract_config<true>();
+    if (rc) return rc;
+    struct KBatch { int T0, nT, max_kb, max_mb; };
+    std::vector<KBatch> batches;
+    const long long per_slot = (long long)2 * E.ne * 32;        // Y doubles per slot of a cluster
+    long long ws = 0, max_ws = 0;
+    for (int T = 0; T < pl->n_clusters; T++) {
+        const ClusterDev &c = pl->cl[T];
+        const long long y = per_slot * c.npad;
+        if (batches.empty() || (ws + y) * (long long)sizeof(double) > WS_BYTES || batches.back().nT == 65535) {
+            batches.push_back({T, 0, 0, 0});
+            ws = 0;
+        }
+        KBatch &b = batches.back();
+        b.nT++;
+        b.max_kb = std::max(b.max_kb, (c.npad + 31) / 32);
+        b.max_mb = std::max(b.max_mb, (3 * c.m + CT - 1) / CT);
+        ws += y;
+        max_ws = std::max(max_ws, ws);
+    }
+    const int nb = (2 * E.ne + CT - 1) / CT;
+    FactArgs A = {pl->d_cl, nullptr, nullptr, pl->Xh, pl->spec, pl->Acal, nullptr};
+    GPRB_CUDA(cudaMallocAsync((void **)&A.Zw, (size_t)max_ws * sizeof(double), st));
+    for (const KBatch &b : batches) {
+        kef_y_kernel<ZI><<<dim3(E.ne, b.nT, b.max_kb), 128, 0, st>>>(A, P, E, b.T0);
+        GPRB_LAUNCHED();
+        kff_contract_kernel<true><<<dim3(b.nT, b.max_mb, nb), 128, CONTRACT_SMEM, st>>>(A, b.T0, O);
+        GPRB_LAUNCHED();
+    }
+    const cudaError_t e = cudaGetLastError();
+    gprb_pool_free(A.Zw, st);
+    GPRB_CUDA(e);
+    return GPRB_OK;
+}
+
+// GPRB_KFF_FACTORED: '0' keeps the pairwise kernels, '1' takes a factored build whenever the pack has a plan (tests on
+// small packs), unset leaves it to the cost model.  The switch governs K_ff and K_ef alike.
+void factored_switch(bool *off, bool *force) {
+    const char *env = getenv("GPRB_KFF_FACTORED");
+    *off = env && env[0] == '0';
+    *force = env && env[0] == '1';
+}
+
+// the pack's atom plan, built on the first call that can use it; NULL when the pack has none
+int pack_plan(gprb_pack *f, cudaStream_t st, gprb_atom_plan **out) {
+    if (!f->plan_tried) {
+        f->plan_tried = true;
+        int rc = build_plan(f, st, &f->plan);
+        if (rc) return rc;
+    }
+    *out = f->plan && f->plan->n_clusters > 0 ? f->plan : nullptr;
+    return GPRB_OK;
+}
+
 }  // namespace
 
 // K_ff + dK/dl of pack f against itself over the full window with one destination (the caller checked that and zeroed K
 // and dK).  *done = false: the pairwise kernel is to run (GPRB_KFF_FACTORED=0, no plan, or the plan does not pay).
-// GPRB_KFF_FACTORED=1 takes the factored path whenever the pack has a plan (tests on small packs).
 int gprb_kff_factored(gprb_pack *f, double p0, double p1, double zeta, int mode, double *K, long long ldk, double *dK,
                       long long lddk, cudaStream_t st, bool *done) {
     *done = false;
-    const char *env = getenv("GPRB_KFF_FACTORED");
-    const bool off = env && env[0] == '0', force = env && env[0] == '1';
+    bool off, force;
+    factored_switch(&off, &force);
     if (off || f->ks != GPRB_MAX_KS || f->n_rows == 0 || mode == GPRB_FF_DIAG) return GPRB_OK;
     const int kind = mode == GPRB_FF_FULL ? 1 : 0;
     if (!force) {
         const double tiles = (double)((f->n_rows + 7) / 8);
         if (128.0 * (kind ? tiles * tiles : 0.5 * tiles * (tiles + 1.0)) < MIN_PAIRWISE_DMMA) return GPRB_OK;
     }
-    if (!f->plan_tried) {
-        f->plan_tried = true;
-        int rc = build_plan(f, st, &f->plan);
-        if (rc) return rc;
-    }
-    gprb_atom_plan *pl = f->plan;
-    if (!pl || pl->n_clusters == 0) return GPRB_OK;
+    gprb_atom_plan *pl = nullptr;
+    int rc = pack_plan(f, st, &pl);
+    if (rc || !pl) return rc;
     if (!force && pl->pairwise_dmma[kind] < MIN_GAIN * pl->factored_dmma[kind]) return GPRB_OK;
     CovParams P = {};
-    int rc = fill_kernel_params(P, GPRB_KERNEL_RBF, p0, p1, zeta);
-    if (rc) return rc;
+    if ((rc = fill_kernel_params(P, GPRB_KERNEL_RBF, p0, p1, zeta))) return rc;
     if ((rc = build_pairs(pl, kind, st))) return rc;
-    rc = P.zi == 2 ? run_batches<2>(pl, pl->lists[kind], P, mode, K, ldk, dK, lddk, st)
-                   : run_batches<0>(pl, pl->lists[kind], P, mode, K, ldk, dK, lddk, st);
+    ContractOut O = {};
+    O.K = K; O.ldk = ldk; O.dK = dK; O.lddk = lddk; O.mode = mode;
+    rc = P.zi == 2 ? run_batches<2>(pl, pl->lists[kind], P, O, st) : run_batches<0>(pl, pl->lists[kind], P, O, st);
+    if (rc) return rc;
+    *done = true;
+    return GPRB_OK;
+}
+
+// K_fe / K_ef + dK/dl of force pack f (full window, one destination, outputs zeroed by the caller; any of the four may be
+// NULL) against energy pack e.  *done = false: the pairwise kernel is to run.
+int gprb_kef_factored(const gprb_pack *e, gprb_pack *f, double p0, double p1, double zeta, double *Kef, long long ld_ef,
+                      double *Kfe, long long ld_fe, double *dKef, long long ld_def, double *dKfe, long long ld_dfe,
+                      cudaStream_t st, bool *done) {
+    *done = false;
+    bool off, force;
+    factored_switch(&off, &force);
+    if (off || f->ks != GPRB_MAX_KS || e->ks != GPRB_MAX_KS || f->n_rows == 0 || e->n_rows == 0) return GPRB_OK;
+    if (!force && 32.0 * (double)((f->n_rows + 7) / 8) * (double)((e->n_rows + 7) / 8) < MIN_PAIRWISE_DMMA) return GPRB_OK;
+    gprb_atom_plan *pl = nullptr;
+    int rc = pack_plan(f, st, &pl);
+    if (rc || !pl) return rc;
+    if (!force) {
+        double pw = 0.0, fa = 0.0;
+        plan_costs_kef(pl->n_clusters, pl->cgrp.data(), pl->cslots.data(), f->n_rows, e->n_rows, e->n_groups, &pw, &fa);
+        if (pw < MIN_GAIN * fa) return GPRB_OK;
+    }
+    CovParams P = {};
+    if ((rc = fill_kernel_params(P, GPRB_KERNEL_RBF, p0, p1, zeta))) return rc;
+    const KefE E = {e->P, e->elep, e->d_row_ptr, e->n_groups};
+    ContractOut O = {};
+    O.K = Kfe; O.ldk = ld_fe; O.dK = dKfe; O.lddk = ld_dfe;
+    O.K2 = Kef; O.ldk2 = ld_ef; O.dK2 = dKef; O.lddk2 = ld_def;
+    O.ne = e->n_groups; O.group_rowsE = e->d_group_rows;
+    rc = P.zi == 2 ? run_kef<2>(pl, E, P, O, st) : run_kef<0>(pl, E, P, O, st);
     if (rc) return rc;
     *done = true;
     return GPRB_OK;

@@ -749,6 +749,12 @@ static int kef_impl(int kernel, const gprb_pack *e, const gprb_pack *f_, double 
     GPRB_CUDA(zero2d(Kef, ld_ef, rows, e->n_groups, st));
     GPRB_CUDA(zero2d(dKef, ld_def, rows, e->n_groups, st));
     if (f->sched_n == 0 || e->n_rows == 0) return GPRB_OK;
+    // RBF with gradient over a whole force pack: the factored build when the pack's rows share atoms (cov_factored.cu)
+    if (kernel == GPRB_KERNEL_RBF && grad && grp_begin == 0 && grp_end == f->n_groups && n_dst == 1) {
+        bool done = false;
+        if ((rc = gprb_kef_factored(e, f, p0, p1, zeta, Kef, ld_ef, Kfe, ld_fe, dKef, ld_def, dKfe, ld_dfe, st, &done))) return rc;
+        if (done) return GPRB_OK;
+    }
     CovParams P = {};
     if ((rc = init_cov_params(P, kernel, p0, p1, zeta, f, e, grp_begin, grp_end))) return rc;
     P.mode = GPRB_FF_FULL;

@@ -69,7 +69,7 @@ int gprb_pack_info(const gprb_pack *p, int *n_groups, int *n_rows, int *d, int *
 long long gprb_pack_pair_count(const gprb_pack *a, int g0, int g1, const gprb_pack *b);
 
 /* ---- atom plan of a force pack (host part; no device needed) -----------------------------------
- * gprb_kff with dK/dl (RBF) over a whole force pack uses the factored build when the pack's rows are
+ * gprb_kff and gprb_kef with dK/dl (RBF) over a whole force pack use the factored build when the pack's rows are
  * copies of a few atoms' descriptors (one row per neighbour atom of every force centre of a structure).
  * gprb_atom_plan_host cuts the groups into clusters of consecutive groups whose distinct rows, keyed by
  * (hash, code), number at most a_max (and at most max_groups groups); a new cluster also starts when a
@@ -80,12 +80,17 @@ long long gprb_pack_pair_count(const gprb_pack *a, int g0, int g1, const gprb_pa
  * with *n_clusters = 0 when one group alone has more than a_max distinct rows.
  * gprb_atom_plan_cost: the DMMA instructions the pairwise kernel and the factored build execute for
  * such a plan (upper != 0: the J >= I group blocks of GPRB_FF_UPPER / SYMMETRIC, else every block);
- * gprb_kff takes the factored build when pairwise >= 2 x factored. */
+ * gprb_kff takes the factored build when pairwise >= 2 x factored.
+ * gprb_atom_plan_cost_kef: the same for gprb_kef with dK/dl of such a force pack (n_rows rows) against an
+ * energy pack of n_energy_rows rows in n_energy_groups groups; gprb_kef takes the factored build on the
+ * same rule. */
 int gprb_atom_plan_host(int n_groups, const int *row_ptr, const unsigned long long *hash, const int *code,
                         const unsigned char *unique, int a_max, int max_groups,
                         int *n_clusters, int *cluster_grp, int *cluster_slots, int *row_slot, int *slot_rep);
 int gprb_atom_plan_cost(int n_clusters, const int *cluster_grp, const int *cluster_slots, int n_rows, int upper,
                         double *pairwise_dmma, double *factored_dmma);
+int gprb_atom_plan_cost_kef(int n_clusters, const int *cluster_grp, const int *cluster_slots, int n_rows,
+                            int n_energy_rows, int n_energy_groups, double *pairwise_dmma, double *factored_dmma);
 
 /* ---- covariance blocks ------------------------------------------------------------------------
  * kernel = GPRB_KERNEL_RBF: p0 = sigma, p1 = l.   GPRB_KERNEL_DOT: p0 = sigma, p1 = sigma0.
